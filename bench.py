@@ -6,7 +6,7 @@ built-in A->B->C reward machine, per-instance Q tables (QLearning lr=1, gamma=.9
 reference driver's learner). One bench "step" = one fused launch of `--iters` lockstep iterations over the whole batch.
 Multi-GPU (`torchrun`, one rank per GPU) shards independent instances: no data-path collective, weak scaling.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--iters T] [--instances N] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--iters T] [--instances N] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (see the keys in main()). Besides the headline it carries: `configs` (every other BASELINE configuration,
 measured in the same run: config 3 on float64 tables, config 2 batched, config 4 sparse-exact / dense-faithful, config 5 with
@@ -51,7 +51,15 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the `configs` block (the other BASELINE configurations)")
     ap.add_argument("--no-call-by-call", action="store_true", help="skip the per-iteration API measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline engine's state (Q tables, slot words, epsilon, episode "
+                         "statistics) for a fixed sample of instances to DIR/<name>.npy; with several ranks, rank 0's instances")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed; it needs --impl b200")
+    return args
 
 
 # name -> (description, BASELINE config, default instances/GPU, default iters/launch, algorithmic bytes per active
@@ -398,7 +406,7 @@ class Runner:
             dist.barrier()
         torch.cuda.synchronize(self.dev)
 
-    def run(self, steps, warmup, e2e_steps, rank0_sampler=None):
+    def run(self, steps, warmup, e2e_steps, rank0_sampler=None, dump_dir=None):
         import torch
         import torch.distributed as dist
 
@@ -423,6 +431,8 @@ class Runner:
         active = eng.total_active_steps() - steps0
         launches = eng.launches - launches0
         mean_live = ((int(eng.tr_work.sum()) - work0) / max(1, self.n_slots * self.iters * steps)) if eng.sparse else None
+        if dump_dir:  # before the e2e window below trains the same engine further
+            dump_outputs(eng, dump_dir)
 
         # ---- end to end: the public API call on HOST (pinned) buffers, copies inside the timed region ----------------
         e2e = None
@@ -472,6 +482,45 @@ class Runner:
                 e2e["seconds"], e2e["active"] = e2e_s_max, e2e_active
         return {"elapsed_ms": elapsed_ms, "per_launch_ms": per_launch_ms, "active": active, "launches": launches, "mean_live": mean_live,
                 "e2e": e2e, "clocks": clocks, "merge_ms_total": merge_total, "n_merges": len(merge_ms), "steps": steps}
+
+
+def dump_outputs(eng, out_dir, budget=48 << 20):
+    """What a caller of Engine.train holds after the last timed step, as DIR/<name>.npy: the Q tables (table dtype), the decoded
+    slot words, epsilon, the running episode return and the episode statistics (integers as exact float64), for a seeded sample
+    of instances sized to keep the files under `budget` bytes (all instances when they fit; shared tables are written whole).
+    The sample depends only on the instance count and the table shape, so runs with the same arguments write the same
+    entries and two builds can be compared file by file. instances.npy holds indices into this engine's own instances: with
+    several ranks only rank 0 writes, and its indices are also the global instance ids."""
+    import numpy as np
+    import torch
+
+    from multiagent_rlrm_b200 import _abi as abi
+    from multiagent_rlrm_b200.engine import STATS_DTYPE
+
+    eng.sync_tables()  # sparse Q(lambda) keeps the live q values in its trace lists until they are written back
+    N, A = eng.N, eng.A
+    shared = bool(eng.cfg.shared_q)
+    q_bytes = eng.q.numel() * eng.q.element_size()
+    per_instance = (0 if shared else q_bytes // N) + 8 + A * 13 * 8  # its tables, its index, 13 float64 entries per agent slot
+    room = budget - 15 * 128 - (q_bytes if shared else 0)  # 15 files, each with a 128-byte .npy header
+    n = min(N, max(1, room // per_instance))
+    idx = np.arange(N) if n == N else np.sort(np.random.default_rng(0).choice(N, size=n, replace=False))
+    it = torch.from_numpy(idx).to(eng.q.device)
+    rows = eng.q.shape[1:]  # per-instance tables are stored instance-major: (N * A, S, 4), or (N, rows, 4) with per-agent machines
+    q = eng.q if shared else eng.q.reshape(N, -1, *rows)[it].reshape(-1, *rows)
+    slot = eng.slot.view(N, A)[it].cpu().numpy().view(np.uint64)
+    stats = eng.stats.view(N, A, 32)[it].cpu().numpy().reshape(-1).view(STATS_DTYPE).reshape(n, A)
+    out = {"instances": idx, "q": q.cpu().numpy(),
+           "epsilon": eng.epsilon.view(N, A)[it].cpu().numpy(), "ep_return": eng.ep_return.view(N, A)[it].cpu().numpy()}
+    for name, shift, mask in (("cell", abi.SLOT_CELL_SHIFT, 0xFFFF), ("agent_steps", abi.SLOT_STEPS_SHIFT, 0xFFFF),
+                              ("timestep", abi.SLOT_TIME_SHIFT, 0xFFFF), ("rm_state", abi.SLOT_RMSTATE_SHIFT, 0xFF),
+                              ("flags", abi.SLOT_FLAGS_SHIFT, 0xFF)):
+        out["slot_" + name] = (slot >> np.uint64(shift)) & np.uint64(mask)
+    for name in STATS_DTYPE.names:
+        out["stats_" + name] = stats[name]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr if arr.dtype in (np.float32, np.float64) else arr.astype(np.float64))
 
 
 def random_gather_peak(eng, block_bytes, reps=5):
@@ -720,7 +769,8 @@ def run_gpu_arm(args):
     # ---- headline ------------------------------------------------------------------------------------------------------
     shared = scenario(args.workload).shared_q
     r = Runner(args.workload, args.instances, args.iters, rank, world, dev, sync_every=64 if shared else 0)
-    res = r.run(args.steps, args.warmup, max(3, args.steps // 2), (lambda: ClockSampler(local_rank)) if rank == 0 else None)
+    res = r.run(args.steps, args.warmup, max(3, args.steps // 2), (lambda: ClockSampler(local_rank)) if rank == 0 else None,
+                dump_dir=args.dump_outputs if rank == 0 else None)
     head = summarise(args.workload, r, res, world, peak, peak_src)
     if not r.sc.shared_q and r.sc.algo != "qlambda":  # per-instance tables read by scattered row / cell-block gathers
         try:

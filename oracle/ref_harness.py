@@ -19,10 +19,10 @@ import sys
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# the live reference: the read-only tree in the build container, else the copy __graft_entry__.build() staged into the
-# git-ignored oracle/_ref/ (it travels to the GPU box with the snapshot so that bench.py can time the real reference there)
-REFERENCE_ROOT = os.environ.get("RLRM_REFERENCE_ROOT") or (
-    "/root/reference" if os.path.isdir("/root/reference/multiagent_rlrm") else os.path.join(_HERE, "_ref"))
+# the original project's source tree (its multiagent_rlrm package, and tests/ for the tests that read the reference's own
+# test files): RLRM_REFERENCE_ROOT, else the copy __graft_entry__.build() stages into the git-ignored oracle/_ref/
+REFERENCE_ROOT = os.environ.get("RLRM_REFERENCE_ROOT") or os.path.join(_HERE, "_ref")
+REFERENCE_MISSING = "needs the original multiagent-rl-rm sources (set RLRM_REFERENCE_ROOT to its checkout)"
 
 
 def reference_available() -> bool:

@@ -13,7 +13,7 @@ GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the live reference tree at /root/reference")
+    config.addinivalue_line("markers", "reference: needs the original multiagent-rl-rm sources (RLRM_REFERENCE_ROOT)")
 
 
 def golden_names():

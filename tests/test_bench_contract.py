@@ -4,6 +4,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 from conftest import ROOT
 
 
@@ -50,3 +52,55 @@ def test_every_bench_workload_compiles_and_is_described():
             continue
         assert name in bench.WORKLOADS, name
         assert entry["dram_bytes_per_active_step"] > 0 and os.path.exists(os.path.join(ROOT, entry["source"])), name
+
+
+@pytest.mark.parametrize("layout", ["per_slot", "per_agent_rm", "shared"])
+def test_dump_outputs_writes_a_fixed_float_sample_within_budget(layout, tmp_path):
+    """bench.py --dump-outputs on each table layout the engine has — one table per agent slot (N*A, S, 4), per-agent machines
+    concatenated per instance (N, rows, 4), one shared table per agent index (A, S, 4), written whole and charged to the budget
+    first — with a stand-in engine on host tensors (the dump only reads the state arrays): float32 / float64 files under the
+    byte budget, the same seeded instance sample every time, and every array equal to the engine's own at every sampled
+    instance, the slot words decoded with the header's field layout."""
+    import types
+
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, ROOT)
+    import bench
+
+    from multiagent_rlrm_b200.engine import STATS_DTYPE
+
+    N, A = (8192, 4) if layout == "shared" else (2048, 2)
+    q_shape = {"per_slot": (N * A, 100, 4), "per_agent_rm": (N, 300, 4), "shared": (A, 100, 4)}[layout]
+    rng = np.random.default_rng(3)
+    fields = {"cell": rng.integers(0, 1 << 16, N * A), "agent_steps": rng.integers(0, 1 << 16, N * A),
+              "timestep": rng.integers(0, 1 << 16, N * A), "rm_state": rng.integers(0, 1 << 8, N * A), "flags": rng.integers(0, 1 << 8, N * A)}
+    words = (fields["cell"] | fields["agent_steps"] << 16 | fields["timestep"] << 32 | fields["rm_state"] << 48
+             | fields["flags"] << 56).astype(np.uint64)  # include/rlrm_b200.h: slot word bit layout
+    stats = np.zeros(N * A, dtype=STATS_DTYPE)
+    for name in STATS_DTYPE.names:
+        stats[name] = rng.integers(0, 1 << 20, N * A).astype(stats.dtype[name]) / (1 if stats.dtype[name].kind == "u" else 8)
+    eng = types.SimpleNamespace(N=N, A=A, cfg=types.SimpleNamespace(shared_q=int(layout == "shared")), sync_tables=lambda: None,
+                                q=torch.from_numpy(rng.random(q_shape, dtype=np.float32)), slot=torch.from_numpy(words.view(np.int64)),
+                                epsilon=torch.from_numpy(rng.random(N * A)), ep_return=torch.from_numpy(rng.random(N * A)),
+                                stats=torch.from_numpy(stats.view(np.uint8).reshape(N * A, 32)))
+    budget = 1 << 20
+    for out in ("a", "b"):
+        bench.dump_outputs(eng, str(tmp_path / out), budget=budget)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == sorted(p.name for p in (tmp_path / "b").iterdir())
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= budget
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    for f in files:
+        assert got[f[:-4]].dtype in (np.float32, np.float64) and np.array_equal(got[f[:-4]], np.load(tmp_path / "b" / f)), f
+    idx = got.pop("instances").astype(np.int64)
+    assert 0 < len(idx) < N and np.all(np.diff(idx) > 0)
+    q = eng.q.numpy()
+    want = {"q": q if layout == "shared" else q.reshape(N, -1, *q_shape[1:])[idx].reshape(-1, *q_shape[1:]),
+            "epsilon": eng.epsilon.numpy().reshape(N, A)[idx], "ep_return": eng.ep_return.numpy().reshape(N, A)[idx]}
+    want.update({"slot_" + k: v.reshape(N, A)[idx] for k, v in fields.items()})
+    want.update({"stats_" + k: stats[k].reshape(N, A)[idx] for k in STATS_DTYPE.names})
+    assert sorted(got) == sorted(want)
+    for k, v in want.items():
+        assert got[k].shape == v.shape and np.array_equal(got[k], v), k

@@ -55,8 +55,17 @@ def _worker(rank, world, port, shared, out_dir):
     dist.destroy_process_group()
 
 
-def _run(shared, tmp_path, port):
-    mp.spawn(_worker, args=(2, port, shared, str(tmp_path)), nprocs=2, join=True)
+def _free_port():
+    """A port nothing listens on now, so that runs sharing a host do not collide on a fixed rendezvous port."""
+    import socket
+
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
+
+def _run(shared, tmp_path):
+    mp.spawn(_worker, args=(2, _free_port(), shared, str(tmp_path)), nprocs=2, join=True)
     return [np.load(os.path.join(tmp_path, f"r{r}.npz")) for r in range(2)]
 
 
@@ -75,7 +84,7 @@ def test_sharded_per_instance_tables_equal_single_process(tmp_path):
     import multiagent_rlrm_b200 as P
     import oracle as O
 
-    parts = _run(False, tmp_path, 29533)
+    parts = _run(False, tmp_path)
     sc = P.scenario_config5(shared=False)
     o = O.Oracle(P.compile_scenario(sc), 37, "f32")
     o.reset()
@@ -92,7 +101,7 @@ def test_shared_learner_replicas_are_averaged_every_k(tmp_path):
     import multiagent_rlrm_b200 as P
     import oracle as O
 
-    parts = _run(True, tmp_path, 29534)
+    parts = _run(True, tmp_path)
     assert np.array_equal(parts[0]["q"], parts[1]["q"])
     assert int(parts[0]["syncs"]) == 5 == int(parts[1]["syncs"])
     # restate the schedule in one process: two replicas, averaged every 8 iterations

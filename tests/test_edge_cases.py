@@ -95,13 +95,12 @@ def test_edge_case_matches_oracle(name, cuda_device):
 
 
 def test_three_agent_oracle_matches_live_reference():
-    """CPU: the oracle on a 3-agent instance equals the live reference (skipped without /root/reference)."""
-    import os
-
-    if not os.path.isdir("/root/reference/multiagent_rlrm"):
-        pytest.skip("needs /root/reference")
+    """CPU: the oracle on a 3-agent instance equals the live reference (skipped without the reference sources)."""
     import oracle as O
     import ref_harness as H
+
+    if not H.reference_available():
+        pytest.skip(H.REFERENCE_MISSING)
 
     sc, _g, _n, _t = edge_scenarios()["fl_3_agents_qrm"]
     ref = H.run_reference(sc.to_dict(), 2, 400)

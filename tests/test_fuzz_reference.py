@@ -1,20 +1,19 @@
-"""CPU, container only (needs the live reference at /root/reference): the seeded random scenarios of test_fuzz_gpu.py,
+"""CPU, needs the original project's sources (ref_harness.REFERENCE_ROOT): the seeded random scenarios of test_fuzz_gpu.py,
 restricted to what the reference can express (its hard-coded 1000-step cap, no shared learner), run through the LIVE
 reference classes (oracle/ref_harness.py, randomness injected) and through the C oracle — traces and final tables must
 agree bit for bit. Together with test_fuzz_gpu.py (CUDA == oracle on the same generator) this extends reference parity
 from the fixed fixtures to option combinations no fixture has."""
-import os
-
 import numpy as np
 import pytest
 
 import multiagent_rlrm_b200 as P
 import oracle as O
+from ref_harness import REFERENCE_MISSING, reference_available
 
 from test_fuzz_gpu import random_scenario
 
 pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not os.path.isdir("/root/reference/multiagent_rlrm"), reason="live reference tree not present")]
+              pytest.mark.skipif(not reference_available(), reason=REFERENCE_MISSING)]
 
 SEEDS = list(range(0, 128, 4))
 

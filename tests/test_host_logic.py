@@ -1,6 +1,6 @@
 """CPU: host-side logic — C-ABI surface (struct layout, exported symbols, loud failure without CUDA), map parsers,
 Reward Machine bookkeeping, encoders, agent plumbing, the table compiler (brute force against the live reference when
-/root/reference is present) and the slip-threshold arithmetic."""
+its sources are present) and the slip-threshold arithmetic."""
 import ctypes as C
 import json
 import os
@@ -16,9 +16,10 @@ from conftest import GOLDEN_DIR, ROOT
 import multiagent_rlrm_b200 as P
 from multiagent_rlrm_b200 import _abi as abi
 from multiagent_rlrm_b200 import maps, tables
+from ref_harness import REFERENCE_MISSING, REFERENCE_ROOT, reference_available
 
 HEADER = os.path.join(ROOT, "include", "rlrm_b200.h")
-HAVE_REF = os.path.isdir("/root/reference/multiagent_rlrm")
+HAVE_REF = reference_available()
 
 
 # ---------------------------------------------------------------------------------------------- C ABI
@@ -124,9 +125,9 @@ def test_emoji_front_ends_round_trip():
     assert P.parse_map_emoji(maps.emoji_from_ascii_rows(rows)) == maps.parse_frozen_lake_rows(rows)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs /root/reference")
+@pytest.mark.skipif(not HAVE_REF, reason=REFERENCE_MISSING)
 def test_emoji_parsers_equal_live_reference():
-    sys.path[:0] = [os.path.join(ROOT, "oracle", "ref_shim"), "/root/reference"]
+    sys.path[:0] = [os.path.join(ROOT, "oracle", "ref_shim"), REFERENCE_ROOT]
     from multiagent_rlrm.environments.frozen_lake.config_frozen_lake import config as fc
     from multiagent_rlrm.environments.office_world.config_office import config as oc
     from multiagent_rlrm.utils.utils import parse_map_emoji, parse_office_world
@@ -324,7 +325,7 @@ def test_slip_thresholds_equal_numpy_searchsorted():
         assert np.array_equal(want, got), probs
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs /root/reference")
+@pytest.mark.skipif(not HAVE_REF, reason=REFERENCE_MISSING)
 @pytest.mark.parametrize("env_name", ["frozen_lake", "office_world"])
 def test_move_tables_equal_reference_apply_action(env_name):
     """Brute force: for every cell and action the compiled next_cell / blocked bit equals what the reference's
@@ -351,7 +352,7 @@ def test_move_tables_equal_reference_apply_action(env_name):
     assert {(i % W, i // W) for i in np.flatnonzero(c.cell_flags & 1)} == hazards
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs /root/reference")
+@pytest.mark.skipif(not HAVE_REF, reason=REFERENCE_MISSING)
 def test_slip_tables_equal_reference_probability_mappings():
     import ref_harness as H
 
@@ -392,13 +393,13 @@ def test_builtin_office_experiments_known_answers():
     assert c.config.n_rm_states == 5 and c.config.rm_final == 4 and c.config.n_events == 4
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs /root/reference")
+@pytest.mark.skipif(not HAVE_REF, reason=REFERENCE_MISSING)
 def test_builtin_office_experiments_equal_live_reference():
     import ast
 
     import ref_harness as H
 
-    H._import_reference()  # puts the stub packages and /root/reference on sys.path
+    H._import_reference()  # puts the stub packages and the reference tree on sys.path
     from multiagent_rlrm.environments.office_world.config_office import config, get_experiment_for_map as ref_get
 
     from multiagent_rlrm_b200.experiments import OPTIMAL, get_experiment_for_map
@@ -411,7 +412,7 @@ def test_builtin_office_experiments_equal_live_reference():
                 continue
             assert list(r["transitions"].items()) == list(m["transitions"].items()), (mp, exp)  # insertion order matters
             assert r["positions"] == m["positions"] and r["description"] == m["description"], (mp, exp)
-    src = open("/root/reference/multiagent_rlrm/environments/office_world/office_main.py").read()
+    src = open(os.path.join(REFERENCE_ROOT, "multiagent_rlrm", "environments", "office_world", "office_main.py")).read()
     node = next(n for n in ast.parse(src).body if isinstance(n, ast.Assign) and getattr(n.targets[0], "id", "") == "OPTIMAL")
     assert ast.literal_eval(node.value) == OPTIMAL
 
@@ -437,7 +438,7 @@ def test_value_iteration_shaping_known_answers():
     assert rm.potentials == {"state0": -(10 + 0.9 * (15 + 0.9 * 20)), "state1": -(15 + 0.9 * 20), "state2": -20, "state3": 0}
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs /root/reference")
+@pytest.mark.skipif(not HAVE_REF, reason=REFERENCE_MISSING)
 def test_potentials_equal_live_reference():
     import contextlib
     import io

@@ -1,4 +1,4 @@
-"""Container only: the REFERENCE's own test files (unchanged, read from /root/reference/tests) run against this repo's host-side
+"""The REFERENCE's own test files (unchanged, read from <ref_harness.REFERENCE_ROOT>/tests) run against this repo's host-side
 drop-in classes, served under the reference's module names by tests/ref_alias/ref_alias_plugin.py. These are the reference tests
 that need no device: reward machine (4 files), spec io / completion / rewards / summary, encoders, agent plumbing, event contexts."""
 import os
@@ -6,15 +6,16 @@ import subprocess
 import sys
 
 import pytest
+from ref_harness import REFERENCE_MISSING, REFERENCE_ROOT
 
-REF_TESTS = "/root/reference/tests"
+REF_TESTS = os.path.join(REFERENCE_ROOT, "tests")
 FILES = ["test_reward_machine.py", "test_reward_machine_api.py", "test_reward_machine_extras.py", "test_reward_machine_shaping.py",
          "test_rmspec_io.py", "test_rmgen_completion.py", "test_rmgen_rewards.py", "test_rmspec_summary.py",
          "test_state_encoder_frozen_lake.py", "test_utils_encoding.py", "test_agent_rl.py", "test_agent_rl_actions.py",
          "test_officeworld_event_context.py", "test_frozenlake_event_context.py"]
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
-pytestmark = [pytest.mark.reference, pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason="live reference tree not present")]
+pytestmark = [pytest.mark.reference, pytest.mark.skipif(not os.path.isdir(REF_TESTS), reason=REFERENCE_MISSING)]
 
 
 def test_reference_host_side_tests_pass_on_the_dropin_classes():
