@@ -272,9 +272,17 @@ extern "C" int rlrm_create(const rlrm_config_t* cfg, const rlrm_tables_t* tb, in
   }
   kp.S4 = (long long)ncell * kp.nQ * 4;
 
+  const bool f32 = !h->f64;  // the specialised kernels exist for float32 tables
+  h->qrm4_fast = (f32 && kp.algo == RLRM_ALGO_QRM && kp.nQ == 4 && kp.n_qrm == 3 && !kp.shared_q && !kp.use_rsh && !kp.random_starts && !kp.per_agent && cfg->learning_rate >= 0.0 &&
+                  !(h->cfg.reserved & 1));
+  for (int j = 0; j < kp.n_qrm; j++)
+    if (!tb->qrm_states || tb->qrm_states[j] != j) h->qrm4_fast = 0;
+
   // pack the tables into one 16-byte aligned blob
   const int sec = kp.per_agent ? kp.A : 1;  // machine-dependent tables have one section per agent
   const int nd = kp.nQ * (kp.nEv + 1) * sec;
+  const int q4_cls = kp.env_kind == RLRM_ENV_FROZEN_LAKE ? 2 : 4;  // train_qrm4_kernel: env-reward classes per event column
+  const int q4_rec = h->qrm4_fast ? (kp.nEv + 1) * q4_cls : 0;
   int off = 0;
   kp.off_phi = off; off = align16(off + sec * 2 * RLRM_MAX_RM_STATES * 8);
   kp.off_rq = off; off = align16(off + nd * 8);
@@ -286,6 +294,9 @@ extern "C" int rlrm_create(const rlrm_config_t* cfg, const rlrm_tables_t* tb, in
   kp.off_delta = off; off = align16(off + nd);
   kp.off_qrm = off; off = align16(off + RLRM_MAX_RM_STATES * sec);
   kp.off_free = off; off = align16(off + (kp.random_starts ? kp.n_free : 0) * 2);
+  kp.off_q4cell = off; off = align16(off + (q4_rec ? ncell : 0) * 2);
+  kp.off_q4rec = off; off = align16(off + q4_rec * 16);
+  kp.off_q4rew = off; off = align16(off + q4_rec * 4 * 8);
   kp.blob_bytes = off;
   if (off > 48 * 1024) {  // every kernel stages the blob in (non-opt-in) dynamic shared memory
     delete h;
@@ -304,17 +315,45 @@ extern "C" int rlrm_create(const rlrm_config_t* cfg, const rlrm_tables_t* tb, in
   memcpy(host + kp.off_delta, tb->delta, nd);
   if (kp.n_qrm > 0 && tb->qrm_states) memcpy(host + kp.off_qrm, tb->qrm_states, kp.per_agent ? (size_t)kp.nQ * sec : (size_t)kp.n_qrm);
   if (kp.random_starts) memcpy(host + kp.off_free, tb->free_cells, (size_t)kp.n_free * 2);
+  if (q4_rec) {  // train_qrm4_kernel's step records; the layout is described at that kernel
+    const int ncol = kp.nEv + 1;
+    uint16_t* q4cell = reinterpret_cast<uint16_t*>(host + kp.off_q4cell);
+    for (int c = 0; c < ncell; c++) {
+      const int col = tb->label[c] == RLRM_EVENT_NONE ? kp.nEv : tb->label[c];
+      q4cell[c] = (uint16_t)(col * q4_cls) | (uint16_t)((tb->cell_flags[c] & 1) << 15);
+    }
+    for (int col = 0; col < ncol; col++)
+      for (int cls = 0; cls < q4_cls; cls++) {
+        // renv as the kernels form it: FrozenLake r.renv = hole_penalty; OfficeWorld __dadd_rn(wall_pen, plant)
+        const double renv = kp.env_kind == RLRM_ENV_FROZEN_LAKE ? (cls ? kp.hole_penalty : 0.0)
+                                                                 : (cls & 1 ? kp.wall_penalty : 0.0) + (cls & 2 ? kp.hole_penalty : 0.0);
+        const int ri = col * q4_cls + cls;
+        float cf[3];
+        uint32_t meta = 0;
+        for (int u = 0; u < 3; u++) {
+          const unsigned d = tb->delta[u * ncol + col];
+          const unsigned un = d == RLRM_NO_TRANSITION ? (unsigned)u : d;
+          cf[u] = (float)(renv + (d == RLRM_NO_TRANSITION ? 0.0 : tb->rcf[u * ncol + col]));
+          meta |= un << (2 * u);
+          if (kp.rm_final >= 0 && (int)un == kp.rm_final) meta |= 1u << (6 + u);
+        }
+        double* rew = reinterpret_cast<double*>(host + kp.off_q4rew) + ri * 4;
+        for (int q = 0; q < 4; q++) {
+          const unsigned d = tb->delta[q * ncol + col];
+          meta |= (d == RLRM_NO_TRANSITION ? (unsigned)q : d) << (12 + 2 * q);
+          rew[q] = renv + (d == RLRM_NO_TRANSITION ? 0.0 : tb->rq[q * ncol + col]);
+        }
+        unsigned char* r = host + kp.off_q4rec + ri * 16;
+        memcpy(r, cf, 12);
+        memcpy(r + 12, &meta, 4);
+      }
+  }
   cudaError_t e = cudaMalloc(&h->d_blob, off);
   if (e == cudaSuccess) e = cudaMemcpy(h->d_blob, host, off, cudaMemcpyHostToDevice);
   delete[] host;
   if (e != cudaSuccess) { delete h; return fail(RLRM_ERR_CUDA, "table upload: %s", cudaGetErrorString(e)); }
   kp.blob = h->d_blob;
   h->smem_bytes = off;
-  const bool f32 = !h->f64;  // the specialised kernels exist for float32 tables
-  h->qrm4_fast = (f32 && kp.algo == RLRM_ALGO_QRM && kp.nQ == 4 && kp.n_qrm == 3 && !kp.shared_q && !kp.use_rsh && !kp.random_starts && !kp.per_agent && cfg->learning_rate >= 0.0 &&
-                  !(h->cfg.reserved & 1));
-  for (int j = 0; j < kp.n_qrm; j++)
-    if (!tb->qrm_states || tb->qrm_states[j] != j) h->qrm4_fast = 0;
   h->qrmn_fast = (f32 && kp.algo == RLRM_ALGO_QRM && (kp.nQ == 3 || kp.nQ == 5) && kp.n_qrm == kp.nQ - 1 && !kp.shared_q && !kp.use_rsh &&
                   !kp.random_starts && !kp.per_agent && cfg->learning_rate >= 0.0 && !(h->cfg.reserved & 1));
   for (int j = 0; j < kp.n_qrm; j++)

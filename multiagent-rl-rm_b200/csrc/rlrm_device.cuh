@@ -39,6 +39,7 @@ struct KP {
   const unsigned char* blob;
   int blob_bytes;
   int off_next, off_flags, off_label, off_delta, off_rq, off_rcf, off_qrm, off_start, off_phi, off_free;
+  int off_q4cell, off_q4rec, off_q4rew;  // train_qrm4_kernel's precomputed step records (see that kernel), empty otherwise
 };
 
 struct Tab {

@@ -13,6 +13,7 @@
 // (agent_step<.., PRE = true>, see rlrm_device.cuh) so that action -> new cell is ALU-only. Measured A/B (profiles/r02c/
 // r02c_prestep_ab.txt): OfficeWorld, where the chain is blocked-check -> slip -> move, gains 0.3-1.4 %; FrozenLake LOSES 0.2-1.5 %
 // (config 3 headline 4.125e10 -> 4.065e10), so it is on for OfficeWorld only. -DRLRM_PRESTEP_ALL=0/1 forces it off / on.
+// train_qrm4_kernel has its own table-driven step and does not use it (see there).
 #ifdef RLRM_PRESTEP_ALL
 #define RLRM_PRESTEP(ENV) (RLRM_PRESTEP_ALL != 0)
 #else
@@ -158,51 +159,82 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
 // qrm_states == [0, 1, 2] (so a static unroll over rows is the reference's update order), per-instance
 // tables, fixed learning rate, no visit counts; anything else takes train_kernel.
 // ------------------------------------------------------------------------------------------------
-struct __align__(32) F8 {
-  float v[8];
-};
-__device__ __forceinline__ F8 ldg256(const float* p) {
-  F8 r;
-  asm volatile("ld.global.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=f"(r.v[0]), "=f"(r.v[1]), "=f"(r.v[2]), "=f"(r.v[3]), "=f"(r.v[4]), "=f"(r.v[5]), "=f"(r.v[6]), "=f"(r.v[7])
-               : "l"(p)
-               : "memory");
-  return r;
-}
-__device__ __forceinline__ void stg256(float* p, const float* v) {
-  asm volatile("st.global.v8.f32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(p), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]),
-               "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7])
-               : "memory");
-}
 __device__ __forceinline__ float sel4(float a, float b, float c, float d, unsigned k) {
   const float lo = (k & 1u) ? b : a, hi = (k & 1u) ? d : c;
   return (k & 2u) ? hi : lo;
 }
-__device__ __forceinline__ void load_block4(const float* Q, unsigned cell, float B[16], float bmax[4]) {
-  const F8 lo = ldg256(Q + (size_t)cell * 16), hi = ldg256(Q + (size_t)cell * 16 + 8);
-#pragma unroll
-  for (int j = 0; j < 8; j++) {
-    B[j] = lo.v[j];
-    B[8 + j] = hi.v[j];
-  }
-#pragma unroll
-  for (int r = 0; r < 4; r++) bmax[r] = fmaxf(fmaxf(B[4 * r], B[4 * r + 1]), fmaxf(B[4 * r + 2], B[4 * r + 3]));
+// 32-bit shared-memory loads from the staged table blob: train_qrm4_kernel keeps the blob's shared-window address in one
+// register and adds section offsets from the parameter block, instead of carrying (or rebuilding) generic table pointers.
+__device__ __forceinline__ unsigned smem_addr() { return (unsigned)__cvta_generic_to_shared(smem_raw); }
+__device__ __forceinline__ unsigned lds_u16(unsigned a) {
+  unsigned short v;
+  asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(a));
+  return v;
 }
+__device__ __forceinline__ double lds_f64(unsigned a) {
+  double v;
+  asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
+  return v;
+}
+__device__ __forceinline__ uint4 lds_v4(unsigned a) {
+  uint4 v;
+  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a));
+  return v;
+}
+// B = the 64-byte block at `blk` if `take`, else unchanged: two predicated 256-bit loads, no branch
+__device__ __forceinline__ void load_block4_if(const float* blk, bool take, float B[16]) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %17, 0;\n\t"
+      "@p ld.global.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%16];\n\t"
+      "@p ld.global.v8.f32 {%8,%9,%10,%11,%12,%13,%14,%15}, [%16+32];\n\t}"
+      : "+f"(B[0]), "+f"(B[1]), "+f"(B[2]), "+f"(B[3]), "+f"(B[4]), "+f"(B[5]), "+f"(B[6]), "+f"(B[7]), "+f"(B[8]), "+f"(B[9]),
+        "+f"(B[10]), "+f"(B[11]), "+f"(B[12]), "+f"(B[13]), "+f"(B[14]), "+f"(B[15])
+      : "l"(blk), "r"((unsigned)take)
+      : "memory");
+}
+// i * A + a of the calling thread from fresh special-register reads: a kernel that needs the slot index only before and after
+// its loop recomputes it rather than holding two registers across the loop (a spill at the register cap)
+__device__ __forceinline__ long long epilogue_slot(const KP& p) {
+  unsigned tx, bx;
+  asm volatile("mov.u32 %0, %%tid.x;" : "=r"(tx));
+  asm volatile("mov.u32 %0, %%ctaid.x;" : "=r"(bx));
+  const long long tid = (long long)bx * TRAIN_BLOCK + tx;
+  return (tid >> p.g_shift) * p.A + (int)(tid & (p.G - 1));
+}
+__device__ __forceinline__ float max4(const float* v) { return fmaxf(fmaxf(v[0], v[1]), fmaxf(v[2], v[3])); }
 
-// STOCH / LEARN / TRACE are compile-time copies of p.stochastic / learn / (trace != nullptr): the loop body is issue-bound,
-// so runtime flag tests and their constant-bank loads are specialised away. n_qrm is 3 on this path.
-// MINB = resident blocks per SM the register allocation is sized for: 7 (72 registers, no spills) when the whole batch
-// fits in 28 warps per SM anyway (BASELINE config 3: 131,072 threads on 148 SMs), 8 (64 registers, 64 B of spills) when
-// there are more threads than that and the extra resident warps pay (config 5: +21 %, config 3 would lose 8 %).
+// STOCH / LEARN / TRACE are compile-time copies of p.stochastic / learn / (trace != nullptr): the loop body is latency- and
+// issue-bound, so runtime flag tests and their constant-bank loads are specialised away. n_qrm is 3 on this path.
+// MINB = resident blocks per SM the register allocation is sized for: 7 (72 registers) when the whole batch fits in 28 warps
+// per SM anyway (BASELINE config 3: 131,072 threads on 148 SMs), 8 (64 registers) when there are more threads than that and
+// the extra resident warps pay (config 5).
+//
+// The env + reward-machine step reads rlrm_create's qrm4 sections (KP::off_q4cell / off_q4rec / off_q4rew) instead of
+// label / cell_flags / delta / rq / rcf. For a cell, q4cell holds its event column times the number of env-reward classes
+// (2 for FrozenLake: 0 or the hole penalty; 4 for OfficeWorld: 0, wall, plant, wall + plant) and the hole / plant flag in
+// bit 15. Column and class select one 16-byte record: the three counterfactual rewards (float)(renv + rcf[u][col]) (rcf
+// counts 0 without a transition) already rounded to float32, and a word with the counterfactual next states un(u) (2 bits
+// each), "un(u) is final" (bits 6..8) and the next RM state of every current state (2 bits each from bit 12). q4rew holds the
+// step reward renv + rq[rm][col] per (record, current state). Host double addition and (float) are the kernel's __dadd_rn
+// and __double2float_rn, so every stored value is bit-identical to evaluating the tables here; the only float64 operation
+// left in the loop is the episode-return sum.
+//
+// Loop shape: the Philox words of iteration t+1 (and the slip threshold index) are computed right after the cell-block fetch
+// of iteration t is issued, in the shadow of that load; the counter depends on t alone and random starts are excluded, so an
+// episode reset in between changes nothing. The fetch is predicated and the same-cell patches of the block are selects, so
+// the update chain and the next selection form one basic block. Every Q store of iteration t precedes the fetch of t+1 in
+// program order: an agent that steps back into the cell it just left must read what it wrote.
 template <int ENV, bool STOCH, bool LEARN, bool TRACE, int MINB>
 __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DState st, unsigned long long t0, int n_iters,
                                                                 unsigned* trace) {
   Tab tb = stage_tables(p);
+  const unsigned sm = smem_addr();
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long i = tid >> p.g_shift;
   const int a = (int)(tid & (p.G - 1));
   const bool valid = (i < st.N) && (a < p.A);
   const long long k = i * p.A + a;
+  const unsigned n_cls = ENV == RLRM_ENV_FROZEN_LAKE ? 2u : 4u;  // env-reward classes per event column
 
   Slot s = {0, 0, 0, 0, 0};
   double eps = 0.0, ep_ret = 0.0, return_sum = 0.0;
@@ -210,18 +242,19 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
   unsigned long long active_steps = 0;
   unsigned episodes = 0, successes = 0, last_length = 0;
   float last_return = 0.f;
-  float B[16], bmax[4];  // carried cell block Q[cell, rm state, action] and its row maxima
+  float B[16];  // carried cell block Q[cell, rm state, action]
 #pragma unroll
   for (int j = 0; j < 16; j++) B[j] = 0.f;
-#pragma unroll
-  for (int j = 0; j < 4; j++) bmax[j] = 0.f;
+  unsigned w[4] = {0u, 0u, 0u, 0u}, sidx = 0u;  // Philox words and slip threshold index of the coming iteration
   if (valid) {
     s = unpack_slot(st.slot[k]);
     eps = st.epsilon[k];
     if (st.ep_return) ep_ret = st.ep_return[k];
     if (st.stats) return_sum = st.stats[k].return_sum;
     Q = st.q + table_base(p, i, a);
-    load_block4(Q, s.cell, B, bmax);
+    load_block4_if(Q + (size_t)s.cell * 16, true, B);
+    RLRM_PHILOX((unsigned)t0, (unsigned)(t0 >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
+    if (STOCH) sidx = slip_index(p, w[3]);
   }
   unsigned long long explore_thr = explore_threshold(eps);
   bool had_episode = false;
@@ -230,58 +263,106 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
     const unsigned long long t = t0 + (unsigned long long)it;
     bool term = true, trunc = true;
     if (valid) {
-      unsigned w[4];
-      RLRM_PHILOX((unsigned)t, (unsigned)(t >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
-      const PreStep ps = RLRM_PRESTEP(ENV) ? pre_step(p, tb, s.cell, w[3], STOCH) : PreStep{0ull, 0u};
       float4 row;
       row.x = sel4(B[0], B[4], B[8], B[12], s.rm);
       row.y = sel4(B[1], B[5], B[9], B[13], s.rm);
       row.z = sel4(B[2], B[6], B[10], B[14], s.rm);
       row.w = sel4(B[3], B[7], B[11], B[15], s.rm);
       const int action = select_action(row, explore_thr, w, !LEARN, p.n_actions);
+      // env.step + check_terminations (agent_step<ENV, STOCH>, table-driven; slip outcomes from KP::slip_nib)
+#define RLRM_Q4_SLIP(x) ((unsigned)(p.slip_nib >> (((x) * 4 + sidx) * 4)) & 0xFu)
+#define RLRM_Q4_NEXT(x) lds_u16(sm + p.off_next + (s.cell * 4 + (x)) * 2)
       const unsigned before = s.cell;
-      Rec r;
-      agent_step<ENV, STOCH, false, RLRM_PRESTEP(ENV)>(p, tb, s, action, w[3], true, r, ps);
-      const bool moved = r.cell != before;
+      const bool active = (s.flags & RLRM_FLAG_ACTIVE) != 0;
+      bool stepped, env_term;
+      unsigned ex, cls, crec;
+      if (ENV == RLRM_ENV_FROZEN_LAKE) {
+        const bool rm_done = (int)s.rm == p.rm_final;  // ma_frozen_lake.py:107-115 (rm_final < 0 never matches)
+        stepped = active && !rm_done;
+        ex = STOCH ? RLRM_Q4_SLIP((unsigned)action) : (unsigned)action;
+        const unsigned nc = RLRM_Q4_NEXT(ex & 3u);
+        if (stepped && ex != RLRM_ACTION_WAIT) s.cell = nc;
+        crec = lds_u16(sm + p.off_q4cell + s.cell * 2);
+        const bool hole = stepped && (crec & 0x8000u);
+        if (hole) s.flags |= RLRM_FLAG_FAIL;
+        cls = hole ? 1u : 0u;
+        s.steps += stepped ? 1u : 0u;
+        s.time++;
+        trunc = ((int)s.steps > p.max_steps) || ((int)s.time > p.max_steps);
+        env_term = trunc || rm_done || (s.flags & RLRM_FLAG_FAIL);
+        if (env_term) s.flags &= ~RLRM_FLAG_ACTIVE;
+      } else {
+        stepped = active;
+        // the wall test and the move both follow from the action alone: two independent table loads
+        const unsigned slipped = STOCH ? RLRM_Q4_SLIP((unsigned)action) : (unsigned)action;
+        const unsigned nb = RLRM_Q4_NEXT((unsigned)action), nc = RLRM_Q4_NEXT(slipped & 3u);
+        const bool blocked = active && nb == s.cell;  // apply_wall_penalty: "wait", no slip draw
+        if (blocked && p.terminate_hit_walls) s.flags |= RLRM_FLAG_FAIL;
+        ex = blocked ? (unsigned)RLRM_ACTION_WAIT : slipped;
+        if (active && ex != RLRM_ACTION_WAIT) s.cell = nc;
+        crec = lds_u16(sm + p.off_q4cell + s.cell * 2);
+        const bool plant = active && (crec & 0x8000u);
+        if (plant && p.terminate_on_plants) s.flags |= RLRM_FLAG_FAIL;
+        cls = (blocked ? 1u : 0u) | (plant ? 2u : 0u);
+        s.steps += active ? 1u : 0u;
+        s.time++;
+        trunc = (int)s.time > p.max_steps;
+        env_term = (s.flags & RLRM_FLAG_FAIL) != 0;
+        if (env_term || trunc) s.flags &= ~RLRM_FLAG_ACTIVE;
+      }
+#undef RLRM_Q4_SLIP
+#undef RLRM_Q4_NEXT
+      // RewardMachine.step + wrapper merge (rm_environment_wrapper.py:57-107) and the counterfactual inputs, one record
+      const unsigned ri = (crec & 0x7FFFu) + cls;
+      const uint4 rec = lds_v4(sm + p.off_q4rec + ri * 16);
+      const double reward = lds_f64(sm + p.off_q4rew + (ri * 4 + s.rm) * 8);
+      s.rm = (rec.w >> (12 + 2 * s.rm)) & 3u;
+      term = env_term || (int)s.rm == p.rm_final;
+      s.flags &= ~(RLRM_FLAG_DONE | RLRM_FLAG_TRUNC | RLRM_FLAG_FIRST);
+      if (term) s.flags |= RLRM_FLAG_DONE;
+      if (trunc) s.flags |= RLRM_FLAG_TRUNC;
+      if (TRACE)
+        trace[(size_t)it * (size_t)(st.N * p.A) + (size_t)k] = (unsigned)action | ((stepped ? ex : 5u) << 3) | (s.cell << 6) |
+                                                             (s.rm << 16) | ((unsigned)term << 21) | ((unsigned)trunc << 22) |
+                                                             ((unsigned)stepped << 23);
+
+      const bool moved = s.cell != before;
       // values the updates overwrite, read before the carried block is replaced
-      const float cur0 = sel4(B[0], B[1], B[2], B[3], (unsigned)action);
-      const float cur1 = sel4(B[4], B[5], B[6], B[7], (unsigned)action);
-      const float cur2 = sel4(B[8], B[9], B[10], B[11], (unsigned)action);
-      if (moved) load_block4(Q, r.cell, B, bmax);  // the carried block becomes the NEXT cell's block
+      float cur[3];
+#pragma unroll
+      for (int u = 0; u < 3; u++) cur[u] = sel4(B[4 * u], B[4 * u + 1], B[4 * u + 2], B[4 * u + 3], (unsigned)action);
+      load_block4_if(Q + (size_t)s.cell * 16, moved, B);  // the carried block becomes the NEXT cell's block
+      // the next iteration's draws, independent of the block in flight
+      {
+        const unsigned long long tn = t + 1ull;
+        RLRM_PHILOX((unsigned)tn, (unsigned)(tn >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
+        if (STOCH) sidx = slip_index(p, w[3]);
+      }
       if (LEARN) {
         // QRM counterfactual experiences (rm_environment_wrapper.py:122-183) applied by update_q (qlearning.py:70-106),
         // in get_all_states()[:-1] order == row order 0..n_qrm-1 on this path. The next state's row maximum comes from
         // the carried block: a different block when the agent moved, else the live one including earlier updates.
-        const int col = r.event == RLRM_EVENT_NONE ? p.nEv : (int)r.event;
+        float bmax[4];
+#pragma unroll
+        for (int r = 0; r < 4; r++) bmax[r] = max4(B + 4 * r);
         float* dst = Q + (size_t)before * 16 + action;  // infos["prev_s"] is the position before the move
+        const float cf[3] = {__uint_as_float(rec.x), __uint_as_float(rec.y), __uint_as_float(rec.z)};
 #pragma unroll
         for (int u = 0; u < 3; u++) {
-          {
-            const unsigned d = tb.delta[u * (p.nEv + 1) + col];
-            const unsigned un = d == RLRM_NO_TRANSITION ? (unsigned)u : d;
-            const double ru = d == RLRM_NO_TRANSITION ? 0.0 : tb.rcf[u * (p.nEv + 1) + col];
-            const bool done = r.env_term || (p.rm_final >= 0 && (int)un == p.rm_final);
-            const float mx = sel4(bmax[0], bmax[1], bmax[2], bmax[3], un);
-            const float cur = u == 0 ? cur0 : (u == 1 ? cur1 : cur2);
-            const float mf = __fmul_rn(done ? 0.0f : 1.0f, mx);
-            const float inner = __fadd_rn(__double2float_rn(__dadd_rn(r.renv, ru)), __fmul_rn(p.gamma_f, mf));
-            const float nv = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur), __fmul_rn(p.lr_f, inner));
-            if (__float_as_uint(nv) != __float_as_uint(cur)) dst[4 * u] = nv;  // a bit-identical value needs no store
-            if (!moved) {  // same cell: the carried block is the one just written
+          const unsigned un = (rec.w >> (2 * u)) & 3u;
+          const bool done = env_term || ((rec.w >> (6 + u)) & 1u);
+          const float mx = sel4(bmax[0], bmax[1], bmax[2], bmax[3], un);
+          const float mf = __fmul_rn(done ? 0.0f : 1.0f, mx);
+          const float inner = __fadd_rn(cf[u], __fmul_rn(p.gamma_f, mf));
+          const float nv = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur[u]), __fmul_rn(p.lr_f, inner));
+          if (__float_as_uint(nv) != __float_as_uint(cur[u])) dst[4 * u] = nv;  // a bit-identical value needs no store
+          // same cell: the carried block is the one just written
 #pragma unroll
-              for (int c = 0; c < 4; c++) B[4 * u + c] = (c == action) ? nv : B[4 * u + c];
-              bmax[u] = fmaxf(fmaxf(B[4 * u], B[4 * u + 1]), fmaxf(B[4 * u + 2], B[4 * u + 3]));
-            }
-          }
+          for (int c = 0; c < 4; c++) B[4 * u + c] = (!moved && c == action) ? nv : B[4 * u + c];
+          if (u < 2) bmax[u] = max4(B + 4 * u);
         }
       }
-      term = r.term;
-      trunc = r.trunc;
-      ep_ret = __dadd_rn(ep_ret, r.reward);
-      if (TRACE)
-        trace[(size_t)it * (size_t)(st.N * p.A) + (size_t)k] = (unsigned)action | (r.executed << 3) | (r.cell << 6) | (r.q << 16) |
-                                                             ((unsigned)r.term << 21) | ((unsigned)r.trunc << 22) |
-                                                             ((unsigned)r.stepped << 23);
+      ep_ret = __dadd_rn(ep_ret, reward);
     }
     // episode over <=> every agent of the instance terminated, or every agent truncated: AND-reduce the two flags
     // (packed in one word) over the instance's lane group with xor shuffles
@@ -299,15 +380,16 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
       ep_ret = 0.0;
       reset_slot<false>(p, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
-      load_block4(Q, s.cell, B, bmax);
+      load_block4_if(Q + (size_t)s.cell * 16, true, B);
     }
   }
   if (valid) {
-    st.slot[k] = pack_slot(s);
-    st.epsilon[k] = eps;
-    if (st.ep_return) st.ep_return[k] = ep_ret;
+    const long long ko = epilogue_slot(p);
+    st.slot[ko] = pack_slot(s);
+    st.epsilon[ko] = eps;
+    if (st.ep_return) st.ep_return[ko] = ep_ret;
     if (st.stats) {
-      rlrm_stats_t z = st.stats[k];
+      rlrm_stats_t z = st.stats[ko];
       z.active_steps += active_steps;
       z.episodes += episodes;
       z.successes += successes;
@@ -316,7 +398,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
         z.last_return = last_return;
         z.last_length = last_length;
       }
-      st.stats[k] = z;
+      st.stats[ko] = z;
     }
   }
 }
