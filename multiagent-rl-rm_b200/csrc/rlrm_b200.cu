@@ -230,10 +230,15 @@ extern "C" int rlrm_create(const rlrm_config_t* cfg, const rlrm_tables_t* tb, in
     kp.slip_thr32[j] = (unsigned)cfg->slip_thr[j];
     kp.slip_cnt = j + 1;
   }
+  for (int j = kp.slip_cnt; j < 3; j++) kp.slip_thr32[j] = 0xFFFFFFFFu;  // padding for slip_index (see there)
   for (int a = 0; a < 4; a++)
     for (int j = 0; j < 4; j++) kp.slip_outcome[a * 4 + j] = cfg->slip_outcome[a][j];
   kp.slip_nib = 0ull;
-  for (int k = 0; k < 16; k++) kp.slip_nib |= (unsigned long long)(kp.slip_outcome[k] & 0xF) << (4 * k);
+  for (int k = 0; k < 16; k++) {
+    // slip_index returns 3 for a draw of 0xFFFFFFFF whatever slip_cnt is; that draw selects outcome slip_cnt
+    const int src = (k & 3) == 3 ? (k & ~3) + kp.slip_cnt : k;
+    kp.slip_nib |= (unsigned long long)(kp.slip_outcome[src] & 0xF) << (4 * k);
+  }
   kp.terminate_on_plants = cfg->terminate_on_plants; kp.terminate_hit_walls = cfg->terminate_hit_walls;
   kp.hole_penalty = cfg->hole_penalty; kp.wall_penalty = cfg->wall_penalty;
   kp.eps_end = cfg->epsilon_end; kp.eps_decay = cfg->epsilon_decay;

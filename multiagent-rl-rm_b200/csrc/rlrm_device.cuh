@@ -264,11 +264,10 @@ struct PreStep {
   unsigned long long nrow;
   unsigned sidx;
 };
+// Index into KP::slip_nib. rlrm_create pads the thresholds past slip_cnt with 0xFFFFFFFF and the nibble of index 3 with the
+// outcome of index slip_cnt, so no slip_cnt test is needed: only k = 0xFFFFFFFF reaches a padded threshold, and then all three.
 __device__ __forceinline__ unsigned slip_index(const KP& p, unsigned k) {
-  unsigned idx = 0;
-#pragma unroll
-  for (int j = 0; j < 3; j++) idx += (j < p.slip_cnt) && (k >= p.slip_thr32[j]);
-  return idx;
+  return (unsigned)(k >= p.slip_thr32[0]) + (unsigned)(k >= p.slip_thr32[1]) + (unsigned)(k >= p.slip_thr32[2]);
 }
 __device__ __forceinline__ PreStep pre_step(const KP& p, const Tab& tb, unsigned cell, unsigned w3, bool stochastic) {
   PreStep ps;

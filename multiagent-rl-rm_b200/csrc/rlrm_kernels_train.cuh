@@ -219,11 +219,15 @@ __device__ __forceinline__ float max4(const float* v) { return fmaxf(fmaxf(v[0],
 // and __double2float_rn, so every stored value is bit-identical to evaluating the tables here; the only float64 operation
 // left in the loop is the episode-return sum.
 //
-// Loop shape: the Philox words of iteration t+1 (and the slip threshold index) are computed right after the cell-block fetch
-// of iteration t is issued, in the shadow of that load; the counter depends on t alone and random starts are excluded, so an
-// episode reset in between changes nothing. The fetch is predicated and the same-cell patches of the block are selects, so
-// the update chain and the next selection form one basic block. Every Q store of iteration t precedes the fetch of t+1 in
-// program order: an agent that steps back into the cell it just left must read what it wrote.
+// Loop shape: an iteration is three regions. (1) select, step, issue the (predicated) fetch of the next cell's block, then
+// the work that does not read it: the Philox words of iteration t+1 and the slip threshold index (the counter depends on t
+// alone and random starts are excluded, so an episode reset in between changes nothing) and the episode-return sum. (2) The
+// episode-end reduction, a warp-wide shuffle outside the per-slot branches. (3) The counterfactual updates, which read the
+// block. ptxas does not move instructions across these region boundaries, so the draws sit between the fetch and the first
+// instruction that waits for it in every instantiation; within one region it would schedule them after the updates where
+// registers are short (the 72-register MINB 7 case). The same-cell patches of the block are selects. Every Q store of
+// iteration t precedes the fetch of t+1 in program order: an agent that steps back into the cell it just left must read
+// what it wrote.
 template <int ENV, bool STOCH, bool LEARN, bool TRACE, int MINB>
 __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DState st, unsigned long long t0, int n_iters,
                                                                 unsigned* trace) {
@@ -238,7 +242,9 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
 
   Slot s = {0, 0, 0, 0, 0};
   double eps = 0.0, ep_ret = 0.0, return_sum = 0.0;
-  float* Q = st.q;
+  // first cell block of this slot's table, counted in 64-byte blocks: 32 bits suffice, as 2^32 blocks are 256 GiB
+  unsigned qblk = 0u;
+#define RLRM_Q4_BLOCK(cell) (st.q + (size_t)(qblk + (cell)) * 16)
   unsigned long long active_steps = 0;
   unsigned episodes = 0, successes = 0, last_length = 0;
   float last_return = 0.f;
@@ -251,8 +257,8 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
     eps = st.epsilon[k];
     if (st.ep_return) ep_ret = st.ep_return[k];
     if (st.stats) return_sum = st.stats[k].return_sum;
-    Q = st.q + table_base(p, i, a);
-    load_block4_if(Q + (size_t)s.cell * 16, true, B);
+    qblk = (unsigned)k * (unsigned)p.ncell;  // table_base(p, i, a) / 16 on this path
+    load_block4_if(RLRM_Q4_BLOCK(s.cell), true, B);
     RLRM_PHILOX((unsigned)t0, (unsigned)(t0 >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
     if (STOCH) sidx = slip_index(p, w[3]);
   }
@@ -262,19 +268,25 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
   for (int it = 0; it < n_iters; it++) {
     const unsigned long long t = t0 + (unsigned long long)it;
     bool term = true, trunc = true;
+    // what the counterfactual updates take from the step
+    int action = 0;
+    unsigned before = 0u;
+    bool env_term = false, moved = false;
+    uint4 rec = make_uint4(0u, 0u, 0u, 0u);
+    float cur[3] = {0.f, 0.f, 0.f};
     if (valid) {
       float4 row;
       row.x = sel4(B[0], B[4], B[8], B[12], s.rm);
       row.y = sel4(B[1], B[5], B[9], B[13], s.rm);
       row.z = sel4(B[2], B[6], B[10], B[14], s.rm);
       row.w = sel4(B[3], B[7], B[11], B[15], s.rm);
-      const int action = select_action(row, explore_thr, w, !LEARN, p.n_actions);
+      action = select_action(row, explore_thr, w, !LEARN, p.n_actions);
       // env.step + check_terminations (agent_step<ENV, STOCH>, table-driven; slip outcomes from KP::slip_nib)
 #define RLRM_Q4_SLIP(x) ((unsigned)(p.slip_nib >> (((x) * 4 + sidx) * 4)) & 0xFu)
 #define RLRM_Q4_NEXT(x) lds_u16(sm + p.off_next + (s.cell * 4 + (x)) * 2)
-      const unsigned before = s.cell;
+      before = s.cell;
       const bool active = (s.flags & RLRM_FLAG_ACTIVE) != 0;
-      bool stepped, env_term;
+      bool stepped;
       unsigned ex, cls, crec;
       if (ENV == RLRM_ENV_FROZEN_LAKE) {
         const bool rm_done = (int)s.rm == p.rm_final;  // ma_frozen_lake.py:107-115 (rm_final < 0 never matches)
@@ -314,7 +326,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
 #undef RLRM_Q4_NEXT
       // RewardMachine.step + wrapper merge (rm_environment_wrapper.py:57-107) and the counterfactual inputs, one record
       const unsigned ri = (crec & 0x7FFFu) + cls;
-      const uint4 rec = lds_v4(sm + p.off_q4rec + ri * 16);
+      rec = lds_v4(sm + p.off_q4rec + ri * 16);
       const double reward = lds_f64(sm + p.off_q4rew + (ri * 4 + s.rm) * 8);
       s.rm = (rec.w >> (12 + 2 * s.rm)) & 3u;
       term = env_term || (int)s.rm == p.rm_final;
@@ -326,49 +338,49 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
                                                              (s.rm << 16) | ((unsigned)term << 21) | ((unsigned)trunc << 22) |
                                                              ((unsigned)stepped << 23);
 
-      const bool moved = s.cell != before;
+      moved = s.cell != before;
       // values the updates overwrite, read before the carried block is replaced
-      float cur[3];
 #pragma unroll
       for (int u = 0; u < 3; u++) cur[u] = sel4(B[4 * u], B[4 * u + 1], B[4 * u + 2], B[4 * u + 3], (unsigned)action);
-      load_block4_if(Q + (size_t)s.cell * 16, moved, B);  // the carried block becomes the NEXT cell's block
+      load_block4_if(RLRM_Q4_BLOCK(s.cell), moved, B);  // the carried block becomes the NEXT cell's block
       // the next iteration's draws, independent of the block in flight
       {
         const unsigned long long tn = t + 1ull;
         RLRM_PHILOX((unsigned)tn, (unsigned)(tn >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
         if (STOCH) sidx = slip_index(p, w[3]);
       }
-      if (LEARN) {
-        // QRM counterfactual experiences (rm_environment_wrapper.py:122-183) applied by update_q (qlearning.py:70-106),
-        // in get_all_states()[:-1] order == row order 0..n_qrm-1 on this path. The next state's row maximum comes from
-        // the carried block: a different block when the agent moved, else the live one including earlier updates.
-        float bmax[4];
-#pragma unroll
-        for (int r = 0; r < 4; r++) bmax[r] = max4(B + 4 * r);
-        float* dst = Q + (size_t)before * 16 + action;  // infos["prev_s"] is the position before the move
-        const float cf[3] = {__uint_as_float(rec.x), __uint_as_float(rec.y), __uint_as_float(rec.z)};
-#pragma unroll
-        for (int u = 0; u < 3; u++) {
-          const unsigned un = (rec.w >> (2 * u)) & 3u;
-          const bool done = env_term || ((rec.w >> (6 + u)) & 1u);
-          const float mx = sel4(bmax[0], bmax[1], bmax[2], bmax[3], un);
-          const float mf = __fmul_rn(done ? 0.0f : 1.0f, mx);
-          const float inner = __fadd_rn(cf[u], __fmul_rn(p.gamma_f, mf));
-          const float nv = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur[u]), __fmul_rn(p.lr_f, inner));
-          if (__float_as_uint(nv) != __float_as_uint(cur[u])) dst[4 * u] = nv;  // a bit-identical value needs no store
-          // same cell: the carried block is the one just written
-#pragma unroll
-          for (int c = 0; c < 4; c++) B[4 * u + c] = (!moved && c == action) ? nv : B[4 * u + c];
-          if (u < 2) bmax[u] = max4(B + 4 * u);
-        }
-      }
       ep_ret = __dadd_rn(ep_ret, reward);
     }
-    // episode over <=> every agent of the instance terminated, or every agent truncated: AND-reduce the two flags
-    // (packed in one word) over the instance's lane group with xor shuffles
+    // episode over <=> every agent of the instance terminated, or every agent truncated: AND-reduce the two flags (packed in
+    // one word) over the instance's lane group with a fixed xor butterfly; a step at a distance of G or more is masked off
     unsigned flags2 = (term ? 1u : 0u) | (trunc ? 2u : 0u);
-    for (int o = 1; o < p.G; o <<= 1) flags2 &= __shfl_xor_sync(0xFFFFFFFFu, flags2, o);
+#pragma unroll
+    for (int o = 1; o < RLRM_MAX_AGENTS; o <<= 1) flags2 &= __shfl_xor_sync(0xFFFFFFFFu, flags2, o) | (o < p.G ? 0u : 3u);
     const bool over = flags2 != 0u;
+    if (LEARN && valid) {
+      // QRM counterfactual experiences (rm_environment_wrapper.py:122-183) applied by update_q (qlearning.py:70-106),
+      // in get_all_states()[:-1] order == row order 0..n_qrm-1 on this path. The next state's row maximum comes from
+      // the carried block: a different block when the agent moved, else the live one including earlier updates.
+      float bmax[4];
+#pragma unroll
+      for (int r = 0; r < 4; r++) bmax[r] = max4(B + 4 * r);
+      float* dst = RLRM_Q4_BLOCK(before) + action;  // infos["prev_s"] is the position before the move
+      const float cf[3] = {__uint_as_float(rec.x), __uint_as_float(rec.y), __uint_as_float(rec.z)};
+#pragma unroll
+      for (int u = 0; u < 3; u++) {
+        const unsigned un = (rec.w >> (2 * u)) & 3u;
+        const bool done = env_term || ((rec.w >> (6 + u)) & 1u);
+        const float mx = sel4(bmax[0], bmax[1], bmax[2], bmax[3], un);
+        const float mf = __fmul_rn(done ? 0.0f : 1.0f, mx);
+        const float inner = __fadd_rn(cf[u], __fmul_rn(p.gamma_f, mf));
+        const float nv = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur[u]), __fmul_rn(p.lr_f, inner));
+        if (__float_as_uint(nv) != __float_as_uint(cur[u])) dst[4 * u] = nv;  // a bit-identical value needs no store
+        // same cell: the carried block is the one just written
+#pragma unroll
+        for (int c = 0; c < 4; c++) B[4 * u + c] = (!moved && c == action) ? nv : B[4 * u + c];
+        if (u < 2) bmax[u] = max4(B + 4 * u);
+      }
+    }
     if (valid && over) {
       episodes++;
       active_steps += s.steps;  // env.agent_steps[agent] of the finished episode
@@ -380,9 +392,10 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
       ep_ret = 0.0;
       reset_slot<false>(p, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
-      load_block4_if(Q + (size_t)s.cell * 16, true, B);
+      load_block4_if(RLRM_Q4_BLOCK(s.cell), true, B);
     }
   }
+#undef RLRM_Q4_BLOCK
   if (valid) {
     const long long ko = epilogue_slot(p);
     st.slot[ko] = pack_slot(s);
