@@ -255,6 +255,18 @@ int rlrm_destroy(rlrm_handle_t* h);
 /* learner hyper-parameters may be changed between calls (the reference mutates attributes in place) */
 int rlrm_set_learner(rlrm_handle_t* h, double learning_rate, double gamma, double lambd);
 
+/* Hyper-parameter sweep: one learner setting for every contiguous group of group_size instances. Instance i (global id
+ * cfg.instance_offset + i, the id the random draws are keyed on) trains with sets[(instance_offset + i) / group_size] and behaves
+ * bit for bit as instance i of a handle created with that setting. epsilon_start is not here: epsilon is per slot state.
+ * n_sets == 0 clears the sweep. RLRM_ERR_UNSUPPORTED on a shared_q handle; RLRM_ERR_ARG for group_size <= 0, and at launch for
+ * a setting with learning_rate < 0 (None) without state.visits or for instances not covered by n_sets * group_size.
+ * rlrm_set_learner fails on a handle with a sweep. */
+typedef struct rlrm_hyper {
+  double learning_rate; /* < 0: None (1 / visits) */
+  double gamma, lambd, epsilon_end, epsilon_decay;
+} rlrm_hyper_t;
+int rlrm_set_sweep(rlrm_handle_t* h, const rlrm_hyper_t* sets, int32_t n_sets, int64_t group_size);
+
 /* RMEnvironmentWrapper.reset (rm_environment_wrapper.py:28-41) -> env.reset (ma_frozen_lake.py:43-94,
  * ma_office.py:77-120): positions, RM state, counters, epsilon decay, Q(lambda) trace wipe.
  * mask: device uint8 [N] selecting instances, or NULL for all. */

@@ -180,6 +180,7 @@ EXPORTED_SYMBOLS = (
     "rlrm_create",
     "rlrm_destroy",
     "rlrm_set_learner",
+    "rlrm_set_sweep",
     "rlrm_reset",
     "rlrm_reset_at",
     "rlrm_select_action",
@@ -201,6 +202,11 @@ EXPORTED_SYMBOLS = (
     "rlrm_stream_sync",
     "rlrm_probe_random_gather",
 )
+
+
+class Hyper(C.Structure):  # rlrm_hyper_t
+    _fields_ = [("learning_rate", C.c_double), ("gamma", C.c_double), ("lambd", C.c_double), ("epsilon_end", C.c_double),
+                ("epsilon_decay", C.c_double)]
 
 
 class SelectReq(C.Structure):  # rlrm_select_req_t

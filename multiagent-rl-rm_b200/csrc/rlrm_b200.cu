@@ -56,6 +56,10 @@ struct rlrm_handle {
   int pipe_ready;
   int f64;        // float64 tables (cfg.table_dtype == RLRM_TABLE_F64): generic kernels instantiated on double
   int max_smem;   // cudaDevAttrMaxSharedMemoryPerBlockOptin of the device
+  Hyp* d_sweep;   // rlrm_set_sweep: one Hyp per setting (device), null = uniform handle
+  int n_sweep;
+  long long sweep_group;
+  int sweep_lr_none;  // some setting has learning_rate = None (needs state.visits)
 };
 
 // run STMT with T = float or double, whichever table type the handle was created for
@@ -91,16 +95,20 @@ extern "C" int rlrm_device_count(void) {
   return n;
 }
 
-static void fill_learner(KP& kp, double lr, double gamma, double lambd) {
-  kp.lr = lr;
-  kp.gamma = gamma;
-  kp.lr_f = (float)lr;
-  kp.one_minus_lr_f = (float)(1.0 - lr);
-  kp.gamma_f = (float)gamma;
-  kp.trace_decay_f = (float)(gamma * lambd);
-  kp.one_minus_lr = 1.0 - lr;
-  kp.trace_decay = gamma * lambd;
+// the one place the learner constants are derived: the handle's uniform settings and every setting of a sweep
+static void fill_learner(Hyp& hp, double lr, double gamma, double lambd, double eps_end, double eps_decay) {
+  hp.lr = lr;
+  hp.gamma = gamma;
+  hp.eps_end = eps_end;
+  hp.eps_decay = eps_decay;
+  hp.lr_f = (float)lr;
+  hp.one_minus_lr_f = (float)(1.0 - lr);
+  hp.gamma_f = (float)gamma;
+  hp.trace_decay_f = (float)(gamma * lambd);
+  hp.one_minus_lr = 1.0 - lr;
+  hp.trace_decay = gamma * lambd;
 }
+static Sweep sweep_of(const rlrm_handle* h) { return Sweep{h->d_sweep, h->sweep_group}; }
 
 // Table CONTENTS are indices the kernels follow without bounds checks: reject anything out of range here, on the host.
 static int validate_tables(const rlrm_config_t* cfg, const rlrm_tables_t* tb) {
@@ -241,8 +249,7 @@ extern "C" int rlrm_create(const rlrm_config_t* cfg, const rlrm_tables_t* tb, in
   }
   kp.terminate_on_plants = cfg->terminate_on_plants; kp.terminate_hit_walls = cfg->terminate_hit_walls;
   kp.hole_penalty = cfg->hole_penalty; kp.wall_penalty = cfg->wall_penalty;
-  kp.eps_end = cfg->epsilon_end; kp.eps_decay = cfg->epsilon_decay;
-  fill_learner(kp, cfg->learning_rate, cfg->gamma, cfg->lambd);
+  fill_learner(kp.h, cfg->learning_rate, cfg->gamma, cfg->lambd, cfg->epsilon_end, cfg->epsilon_decay);
   kp.decay_on_reset = cfg->decay_on_reset; kp.shared_q = cfg->shared_q;
   {
     const char* e = getenv("RLRM_SHARED_BALANCED");  // tuning switch, see shared_train_kernel
@@ -380,13 +387,15 @@ extern "C" int rlrm_create(const rlrm_config_t* cfg, const rlrm_tables_t* tb, in
   if (h->qrmb_fast) {  // opt in to the device maximum (per function, only ever raised)
     cudaError_t e2 = cudaSuccess;
 #define RLRM_OPTIN(K) if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(K, cudaFuncAttributeMaxDynamicSharedMemorySize, h->max_smem)
-#define RLRM_OPTIN_T(T, M)                                                                                                                             \
-    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 3, T, M>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 3, T, M>));          \
-    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 7, T, M>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 11, T, M>));         \
-    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 15, T, M>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 7, T, M>));        \
-    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 11, T, M>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 15, T, M>))
-    if (h->f64) { if (h->qrmb_tma) { RLRM_OPTIN_T(double, true); } else { RLRM_OPTIN_T(double, false); } }
-    else { if (h->qrmb_tma) { RLRM_OPTIN_T(float, true); } else { RLRM_OPTIN_T(float, false); } }
+#define RLRM_OPTIN_T(T, M, SW)                                                                                                                             \
+    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 3, T, M, SW>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 3, T, M, SW>));          \
+    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 7, T, M, SW>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 11, T, M, SW>));         \
+    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_FROZEN_LAKE, 15, T, M, SW>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 7, T, M, SW>));        \
+    RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 11, T, M, SW>)); RLRM_OPTIN((train_qrm_block_kernel<RLRM_ENV_OFFICE_WORLD, 15, T, M, SW>))
+#define RLRM_OPTIN_TS(T, M) RLRM_OPTIN_T(T, M, false); RLRM_OPTIN_T(T, M, true)  /* uniform and sweep instantiations */
+    if (h->f64) { if (h->qrmb_tma) { RLRM_OPTIN_TS(double, true); } else { RLRM_OPTIN_TS(double, false); } }
+    else { if (h->qrmb_tma) { RLRM_OPTIN_TS(float, true); } else { RLRM_OPTIN_TS(float, false); } }
+#undef RLRM_OPTIN_TS
 #undef RLRM_OPTIN_T
 #undef RLRM_OPTIN
     if (e2 != cudaSuccess) h->qrmb_fast = 0;
@@ -458,6 +467,7 @@ extern "C" int rlrm_destroy(rlrm_handle_t* h) {
   cudaSetDevice(h->device);
   if (h->d_blob) cudaFree(h->d_blob);
   if (h->d_coop) cudaFree(h->d_coop);
+  if (h->d_sweep) cudaFree(h->d_sweep);
   if (h->pipe_ready) {
     for (int k = 0; k < 2; k++) cudaStreamDestroy(h->pipe_stream[k]);
     for (int k = 0; k < 3 * 8; k++) cudaEventDestroy(h->pipe_event[k]);
@@ -468,9 +478,44 @@ extern "C" int rlrm_destroy(rlrm_handle_t* h) {
 
 extern "C" int rlrm_set_learner(rlrm_handle_t* h, double learning_rate, double gamma, double lambd) {
   if (!h) return fail(RLRM_ERR_ARG, "null handle");
+  if (h->d_sweep) return fail(RLRM_ERR_UNSUPPORTED, "rlrm_set_learner on a sweep handle: change the settings with rlrm_set_sweep");
   h->cfg.learning_rate = learning_rate; h->cfg.gamma = gamma; h->cfg.lambd = lambd;
-  fill_learner(h->kp, learning_rate, gamma, lambd);
+  fill_learner(h->kp.h, learning_rate, gamma, lambd, h->kp.h.eps_end, h->kp.h.eps_decay);
   if (learning_rate < 0.0) h->qrm4_fast = h->ql_fast = h->qrmn_fast = h->qrmb_fast = 0;
+  return RLRM_OK;
+}
+
+extern "C" int rlrm_set_sweep(rlrm_handle_t* h, const rlrm_hyper_t* sets, int32_t n_sets, int64_t group_size) {
+  if (!h) return fail(RLRM_ERR_ARG, "null handle");
+  if (n_sets < 0 || (n_sets > 0 && !sets)) return fail(RLRM_ERR_ARG, "rlrm_set_sweep: bad settings list");
+  if (n_sets > 0 && h->cfg.shared_q) return fail(RLRM_ERR_UNSUPPORTED, "rlrm_set_sweep: instances of a shared table share one learner");
+  if (n_sets > 0 && group_size <= 0) return fail(RLRM_ERR_ARG, "rlrm_set_sweep: group_size must be positive");
+  CUDA_TRY(cudaSetDevice(h->device));
+  Hyp* d = nullptr;
+  int lr_none = 0;
+  if (n_sets > 0) {
+    Hyp* host = new (std::nothrow) Hyp[n_sets];
+    if (!host) return fail(RLRM_ERR_ARG, "out of host memory");
+    for (int g = 0; g < n_sets; g++) {
+      fill_learner(host[g], sets[g].learning_rate, sets[g].gamma, sets[g].lambd, sets[g].epsilon_end, sets[g].epsilon_decay);
+      lr_none |= sets[g].learning_rate < 0.0;
+    }
+    cudaError_t e = cudaMalloc(&d, (size_t)n_sets * sizeof(Hyp));
+    if (e == cudaSuccess) e = cudaMemcpy(d, host, (size_t)n_sets * sizeof(Hyp), cudaMemcpyHostToDevice);
+    delete[] host;
+    if (e != cudaSuccess) {
+      if (d) cudaFree(d);
+      return fail(RLRM_ERR_CUDA, "rlrm_set_sweep: upload: %s", cudaGetErrorString(e));
+    }
+  }
+  if (h->d_sweep) {
+    CUDA_TRY(cudaDeviceSynchronize());  // launches already queued may still read the old settings
+    cudaFree(h->d_sweep);
+  }
+  h->d_sweep = d;
+  h->n_sweep = n_sets;
+  h->sweep_group = n_sets > 0 ? group_size : 0;
+  h->sweep_lr_none = lr_none;
   return RLRM_OK;
 }
 
@@ -509,7 +554,10 @@ static int check_state(const rlrm_handle_t* h, const rlrm_state_t* st, bool need
     if (st->tr_cap < h->cfg.max_steps + 1) return fail(RLRM_ERR_ARG, "tr_cap must be >= max_steps + 1");
     if (h->kp.S4 > 65535) return fail(RLRM_ERR_UNSUPPORTED, "sparse traces need S*4 <= 65535");
   }
-  if (need_q && h->cfg.learning_rate < 0 && !st->visits) return fail(RLRM_ERR_ARG, "learning_rate=None needs state.visits");
+  if (need_q && (h->d_sweep ? h->sweep_lr_none : h->cfg.learning_rate < 0) && !st->visits)
+    return fail(RLRM_ERR_ARG, "learning_rate=None needs state.visits");
+  if (h->d_sweep && (long long)h->kp.instance_offset + st->n_instances > (long long)h->n_sweep * h->sweep_group)
+    return fail(RLRM_ERR_ARG, "the sweep's settings do not cover instances [instance_offset, instance_offset + n_instances)");
   if (need_q && h->cfg.shared_q && h->cfg.learning_rate < 0) return fail(RLRM_ERR_UNSUPPORTED, "shared table with learning_rate=None");
   if (need_q && h->cfg.shared_q && (!st->acc_sum || !st->acc_cnt || !st->acc_last))
     return fail(RLRM_ERR_ARG, "shared_q needs state.acc_sum / acc_cnt / acc_last");
@@ -536,7 +584,7 @@ extern "C" int rlrm_reset_at(rlrm_handle_t* h, const rlrm_state_t* st, const uin
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
   const long long n = st->n_instances * h->kp.A;
-  reset_kernel<<<blocks_for(n, 256), 256, h->smem_bytes, s>>>(h->kp, dstate(st), mask, t);
+  reset_kernel<<<blocks_for(n, 256), 256, h->smem_bytes, s>>>(h->kp, dstate(st), mask, t, sweep_of(h));
   LAUNCH_CHECK(h);
   if (h->cfg.algo == RLRM_ALGO_QLAMBDA && st->e) {
     RLRM_BY_T(h, clear_traces_kernel<T><<<blocks_for(st->n_instances * ((h->kp.per_agent ? h->kp.sum4 : (long long)h->kp.A * h->kp.S4) / 4), 256), 256, 0, s>>>(h->kp, dstate(st), mask));
@@ -673,8 +721,8 @@ extern "C" int rlrm_update(rlrm_handle_t* h, const rlrm_state_t* st, const uint1
   if (h->kp.algo == RLRM_ALGO_QLAMBDA && !st->e)
     return fail(RLRM_ERR_UNSUPPORTED, "rlrm_update on Q(lambda) needs dense traces (state.e); sparse traces are for rlrm_train");
   if (h->kp.algo == RLRM_ALGO_QLAMBDA)
-    RLRM_BY_T(h, update_qlambda_kernel<T><<<(unsigned)n, 256, 0, s>>>(h->kp, dstate(st), obs_cell, actions, term_arg, dout(out)));
-#define RLRM_UPD(ALGO, PA) RLRM_BY_T(h, update_kernel<ALGO, PA, T><<<blocks_for(n, 256), 256, h->smem_bytes, s>>>(h->kp, dstate(st), obs_cell, actions, term_arg, dout(out)))
+    RLRM_BY_T(h, update_qlambda_kernel<T><<<(unsigned)n, 256, 0, s>>>(h->kp, dstate(st), obs_cell, actions, term_arg, dout(out), sweep_of(h)));
+#define RLRM_UPD(ALGO, PA) RLRM_BY_T(h, update_kernel<ALGO, PA, T><<<blocks_for(n, 256), 256, h->smem_bytes, s>>>(h->kp, dstate(st), obs_cell, actions, term_arg, dout(out), sweep_of(h)))
   else if (h->kp.algo == RLRM_ALGO_QRM) {
     if (h->kp.per_agent) RLRM_UPD(RLRM_ALGO_QRM, true); else RLRM_UPD(RLRM_ALGO_QRM, false);
   } else {
@@ -689,29 +737,31 @@ extern "C" int rlrm_update(rlrm_handle_t* h, const rlrm_state_t* st, const uint1
   return RLRM_OK;
 }
 
-template <int ENV>
+// SWEEP: the handle has per-group settings (h->d_sweep); every family takes them in its own kernel, fast paths included
+template <int ENV, bool SWEEP>
 static void launch_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, int n_iters, int learn, uint32_t* trace, cudaStream_t s,
                          double* reward_out = nullptr) {
   const KP& kp = h->kp;
+  const Sweep sw = sweep_of(h);
   const bool fast_ok = reward_out == nullptr;  // the per-step reward output exists in the generic kernels only
   if (kp.algo == RLRM_ALGO_QLAMBDA && !st->e) {
     const long long ipw = 32 / (kp.qls_lg << kp.g_shift);  // instances per warp
     const long long qls_warps = (st->n_instances + ipw - 1) / ipw;
-    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, true><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out));
-    else RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, false><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out));
+    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, true, SWEEP><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
+    else RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, false, SWEEP><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
   } else if (kp.algo == RLRM_ALGO_QLAMBDA) {
-    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_kernel<ENV, T, true><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out));
-    else RLRM_BY_T(h, train_qlambda_kernel<ENV, T, false><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out));
+    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_kernel<ENV, T, true, SWEEP><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
+    else RLRM_BY_T(h, train_qlambda_kernel<ENV, T, false, SWEEP><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
   } else {
     const long long threads = st->n_instances * kp.G;
     const unsigned grid = blocks_for(threads, TRAIN_BLOCK);
-#define RLRM_TRAIN(ALGO, PA) RLRM_BY_T(h, train_kernel<ENV, ALGO, PA, T><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out))
+#define RLRM_TRAIN(ALGO, PA) RLRM_BY_T(h, train_kernel<ENV, ALGO, PA, T, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw))
     if (fast_ok && kp.algo == RLRM_ALGO_QRM && h->qrm4_fast && !st->visits) {
       const DState d = dstate(st);
 #define RLRM_QRM4(ST, LE, TR)                                                                                          \
   do {                                                                                                                \
-    if (dense_batch) train_qrm4_kernel<ENV, ST, LE, TR, 8><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace); \
-    else train_qrm4_kernel<ENV, ST, LE, TR, 7><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace);   \
+    if (dense_batch) train_qrm4_kernel<ENV, ST, LE, TR, 8, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace, sw); \
+    else train_qrm4_kernel<ENV, ST, LE, TR, 7, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace, sw);   \
   } while (0)
       // more threads than 7 resident blocks per SM hold: take the 64-register instantiation (8 blocks per SM)
       const bool dense_batch = threads > (long long)h->num_sms * 7 * TRAIN_BLOCK;
@@ -732,8 +782,8 @@ static void launch_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, 
       const DState d = dstate(st);
 #define RLRM_QRMN(ST, LE, TR)                                                                                             \
   do {                                                                                                                   \
-    if (kp.nQ == 3) train_qrmn_kernel<ENV, 3, ST, LE, TR><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace); \
-    else train_qrmn_kernel<ENV, 5, ST, LE, TR><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace);       \
+    if (kp.nQ == 3) train_qrmn_kernel<ENV, 3, ST, LE, TR, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace, sw); \
+    else train_qrmn_kernel<ENV, 5, ST, LE, TR, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace, sw);       \
   } while (0)
       const int key = (kp.stochastic ? 4 : 0) | (learn ? 2 : 0) | (trace ? 1 : 0);
       switch (key) {
@@ -752,17 +802,17 @@ static void launch_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, 
       const DState d = dstate(st);
 #define RLRM_QRMB(M)                                                                                                                       \
   do {                                                                                                                                   \
-    if (kp.n_qrm <= 3) RLRM_BY_T(h, train_qrm_block_kernel<ENV, 3, T, M><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace));        \
-    else if (kp.n_qrm <= 7) RLRM_BY_T(h, train_qrm_block_kernel<ENV, 7, T, M><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace));   \
-    else if (kp.n_qrm <= 11) RLRM_BY_T(h, train_qrm_block_kernel<ENV, 11, T, M><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace)); \
-    else RLRM_BY_T(h, train_qrm_block_kernel<ENV, 15, T, M><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace));                     \
+    if (kp.n_qrm <= 3) RLRM_BY_T(h, train_qrm_block_kernel<ENV, 3, T, M, SWEEP><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace, sw));        \
+    else if (kp.n_qrm <= 7) RLRM_BY_T(h, train_qrm_block_kernel<ENV, 7, T, M, SWEEP><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace, sw));   \
+    else if (kp.n_qrm <= 11) RLRM_BY_T(h, train_qrm_block_kernel<ENV, 11, T, M, SWEEP><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace, sw)); \
+    else RLRM_BY_T(h, train_qrm_block_kernel<ENV, 15, T, M, SWEEP><<<grid, TRAIN_BLOCK, h->qrmb_smem, s>>>(kp, d, t0, n_iters, learn, trace, sw));                     \
   } while (0)
       if (h->qrmb_tma) RLRM_QRMB(true); else RLRM_QRMB(false);
 #undef RLRM_QRMB
     }
     else if (fast_ok && kp.algo == RLRM_ALGO_QL && h->ql_fast && !st->visits) {
       const DState d = dstate(st);
-#define RLRM_QLF(ST, LE, TR) train_ql_fast_kernel<ENV, ST, LE, TR><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace)
+#define RLRM_QLF(ST, LE, TR) train_ql_fast_kernel<ENV, ST, LE, TR, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, d, t0, n_iters, trace, sw)
       const int key = (kp.stochastic ? 4 : 0) | (learn ? 2 : 0) | (trace ? 1 : 0);
       switch (key) {
         case 0: RLRM_QLF(false, false, false); break;
@@ -844,8 +894,8 @@ extern "C" int rlrm_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0,
           if (h->kp.algo == RLRM_ALGO_QRM) shared_propose_kernel<RLRM_ENV_OFFICE_WORLD, RLRM_ALGO_QRM><<<grid, SHARED_BLOCK, h->shared_smem_bytes, s>>>(h->kp, d, t0 + it, learn, tr);
           else shared_propose_kernel<RLRM_ENV_OFFICE_WORLD, RLRM_ALGO_QL><<<grid, SHARED_BLOCK, h->shared_smem_bytes, s>>>(h->kp, d, t0 + it, learn, tr);
         }
-      } else if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) launch_train<RLRM_ENV_FROZEN_LAKE>(h, st, t0 + it, 1, learn, tr, s);
-      else launch_train<RLRM_ENV_OFFICE_WORLD>(h, st, t0 + it, 1, learn, tr, s);
+      } else if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) launch_train<RLRM_ENV_FROZEN_LAKE, false>(h, st, t0 + it, 1, learn, tr, s);
+      else launch_train<RLRM_ENV_OFFICE_WORLD, false>(h, st, t0 + it, 1, learn, tr, s);
       LAUNCH_CHECK(h);
       if (learn) {
         apply_shared_kernel<<<blocks_for(h->kp.per_agent ? h->kp.sum4 : (long long)h->kp.A * h->kp.S4, 256), 256, 0, s>>>(h->kp, dstate(st));
@@ -854,8 +904,13 @@ extern "C" int rlrm_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0,
     }
     return RLRM_OK;
   }
-  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) launch_train<RLRM_ENV_FROZEN_LAKE>(h, st, t0, n_iters, learn, trace, s);
-  else launch_train<RLRM_ENV_OFFICE_WORLD>(h, st, t0, n_iters, learn, trace, s);
+  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) {
+    if (h->d_sweep) launch_train<RLRM_ENV_FROZEN_LAKE, true>(h, st, t0, n_iters, learn, trace, s);
+    else launch_train<RLRM_ENV_FROZEN_LAKE, false>(h, st, t0, n_iters, learn, trace, s);
+  } else {
+    if (h->d_sweep) launch_train<RLRM_ENV_OFFICE_WORLD, true>(h, st, t0, n_iters, learn, trace, s);
+    else launch_train<RLRM_ENV_OFFICE_WORLD, false>(h, st, t0, n_iters, learn, trace, s);
+  }
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }
@@ -991,8 +1046,13 @@ extern "C" int rlrm_iterate(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t
   }
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) launch_train<RLRM_ENV_FROZEN_LAKE>(h, st, t, 1, learn, record, s, reward);
-  else launch_train<RLRM_ENV_OFFICE_WORLD>(h, st, t, 1, learn, record, s, reward);
+  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) {
+    if (h->d_sweep) launch_train<RLRM_ENV_FROZEN_LAKE, true>(h, st, t, 1, learn, record, s, reward);
+    else launch_train<RLRM_ENV_FROZEN_LAKE, false>(h, st, t, 1, learn, record, s, reward);
+  } else {
+    if (h->d_sweep) launch_train<RLRM_ENV_OFFICE_WORLD, true>(h, st, t, 1, learn, record, s, reward);
+    else launch_train<RLRM_ENV_OFFICE_WORLD, false>(h, st, t, 1, learn, record, s, reward);
+  }
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }
@@ -1013,7 +1073,7 @@ static int update_list_impl(rlrm_handle_t* h, const rlrm_state_t* st, int64_t sl
     sa.state = sel->state; sa.best = sel->best; sa.epsilon = sel->epsilon; sa.seq = sel->seq;
     for (int j = 0; j < 4; j++) sa.draws[j] = sel->draws[j];
   }
-  RLRM_BY_T(h, update_list_kernel<T><<<1, (h->kp.algo == RLRM_ALGO_QLAMBDA && n > 0) ? 256 : 32, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), slot, n, experiences, sel, sa));
+  RLRM_BY_T(h, update_list_kernel<T><<<1, (h->kp.algo == RLRM_ALGO_QLAMBDA && n > 0) ? 256 : 32, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), slot, n, experiences, sel, sa, sweep_of(h)));
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }

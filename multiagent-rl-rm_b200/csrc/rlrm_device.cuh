@@ -9,6 +9,20 @@
 // ------------------------------------------------------------------------------------------------
 // kernel parameter block (passed by value)
 // ------------------------------------------------------------------------------------------------
+// Learner hyper-parameters and the constants derived from them on the host (fill_learner). Every kernel reads them as KP::h;
+// a sweep handle (rlrm_set_sweep) owns a device array of them, one per setting, which apply_sweep loads into a kernel's copy.
+struct Hyp {
+  double lr, gamma, eps_end, eps_decay;
+  float lr_f, one_minus_lr_f, gamma_f, trace_decay_f;  // (float)lr, (float)(1-lr), (float)gamma, (float)(gamma*lambda)
+  double one_minus_lr, trace_decay;                    // 1 - lr and gamma*lambda as doubles (float64 tables)
+};
+// The settings of a sweep handle: instance i (global id instance_offset + i) trains with hyp[(instance_offset + i) / group].
+// Passed as the LAST kernel argument, so the parameter offsets of everything before it are those of a uniform launch.
+struct Sweep {
+  const Hyp* hyp;  // null: uniform handle
+  long long group;
+};
+
 struct KP {
   int env_kind, driver, algo;
   int A, G, g_shift;  // agents, lane-group size (power of two >= A), log2(G)
@@ -21,9 +35,7 @@ struct KP {
   unsigned long long slip_nib;  // slip_outcome as 16 nibbles: outcome of (intended a, threshold index k) at bits 4*(4a+k)
   int terminate_on_plants, terminate_hit_walls;
   double hole_penalty, wall_penalty;
-  double lr, gamma, eps_end, eps_decay;
-  float lr_f, one_minus_lr_f, gamma_f, trace_decay_f;  // (float)lr, (float)(1-lr), (float)gamma, (float)(gamma*lambda)
-  double one_minus_lr, trace_decay;                    // 1 - lr and gamma*lambda as doubles (float64 tables)
+  Hyp h;  // same place and layout as the fields it groups, so uniform kernels address the constant bank as before
   int decay_on_reset, shared_q, use_rsh, random_starts, n_free;
   int shared_balanced;  // shared_train_kernel: contiguous equal chunks per block (1) or grid-stride (0)
   int qls_lg;           // train_qlambda_sparse_kernel: lanes per agent (power of two, 4 .. 32 / G)
@@ -135,10 +147,10 @@ struct RT<float> {
   static __device__ __forceinline__ float sub(float a, float b) { return __fsub_rn(a, b); }
   static __device__ __forceinline__ float cvt(double x) { return __double2float_rn(x); }
   static __device__ __forceinline__ bool same_bits(float a, float b) { return __float_as_uint(a) == __float_as_uint(b); }
-  static __device__ __forceinline__ float lr(const KP& p) { return p.lr_f; }
-  static __device__ __forceinline__ float one_minus_lr(const KP& p) { return p.one_minus_lr_f; }
-  static __device__ __forceinline__ float gamma(const KP& p) { return p.gamma_f; }
-  static __device__ __forceinline__ float decay(const KP& p) { return p.trace_decay_f; }
+  static __device__ __forceinline__ float lr(const KP& p) { return p.h.lr_f; }
+  static __device__ __forceinline__ float one_minus_lr(const KP& p) { return p.h.one_minus_lr_f; }
+  static __device__ __forceinline__ float gamma(const KP& p) { return p.h.gamma_f; }
+  static __device__ __forceinline__ float decay(const KP& p) { return p.h.trace_decay_f; }
   static __device__ __forceinline__ row_t zero_row() { return make_float4(0.f, 0.f, 0.f, 0.f); }
   static __device__ __forceinline__ pair_t make_pair(float a, float b) { return make_float2(a, b); }
 };
@@ -151,10 +163,10 @@ struct RT<double> {
   static __device__ __forceinline__ double sub(double a, double b) { return __dsub_rn(a, b); }
   static __device__ __forceinline__ double cvt(double x) { return x; }
   static __device__ __forceinline__ bool same_bits(double a, double b) { return __double_as_longlong(a) == __double_as_longlong(b); }
-  static __device__ __forceinline__ double lr(const KP& p) { return p.lr; }
-  static __device__ __forceinline__ double one_minus_lr(const KP& p) { return p.one_minus_lr; }
-  static __device__ __forceinline__ double gamma(const KP& p) { return p.gamma; }
-  static __device__ __forceinline__ double decay(const KP& p) { return p.trace_decay; }
+  static __device__ __forceinline__ double lr(const KP& p) { return p.h.lr; }
+  static __device__ __forceinline__ double one_minus_lr(const KP& p) { return p.h.one_minus_lr; }
+  static __device__ __forceinline__ double gamma(const KP& p) { return p.h.gamma; }
+  static __device__ __forceinline__ double decay(const KP& p) { return p.h.trace_decay; }
   static __device__ __forceinline__ row_t zero_row() { return double4r{0.0, 0.0, 0.0, 0.0}; }
   static __device__ __forceinline__ pair_t make_pair(double a, double b) { return make_double2(a, b); }
 };
@@ -390,7 +402,7 @@ __device__ __forceinline__ void update_q(const KP& p, T* Q, unsigned* V, unsigne
   const T mf = R::mul(terminated ? (T)0 : (T)1, mx);
   const T inner = R::add(R::cvt(r), R::mul(R::gamma(p), mf));
   T out;
-  if (p.lr < 0.0) {  // lr = 1/visits is an np.float64: the outer expression is evaluated in double
+  if (p.h.lr < 0.0) {  // lr = 1/visits is an np.float64: the outer expression is evaluated in double
     const unsigned v = V[s * 4 + a] + 1;
     V[s * 4 + a] = v;
     const double lr = __ddiv_rn(1.0, (double)v);
@@ -434,12 +446,12 @@ __device__ __forceinline__ void agent_update(const KP& p, const Tab& tb, T* Q, u
       const double ru = d == RLRM_NO_TRANSITION ? 0.0 : tb.rcf[u * (p.nEv + 1) + col];
       const bool done = r.env_term || (p.rm_final >= 0 && (int)un == p.rm_final);
       double rew = __dadd_rn(r.renv, ru);
-      if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.gamma, tb.phi[un]), tb.phi[u]));  // qlearning.py:93-105
+      if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.h.gamma, tb.phi[un]), tb.phi[u]));  // qlearning.py:93-105
       update_q(p, Q, V, r.prev_cell * p.nQ + u, action, rew, r.cell * p.nQ + un, done, acc);
     }
   } else {
     double rew = r.reward;
-    if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.gamma, tb.phi[p.phi_row + r.q]), tb.phi[p.phi_row + r.prev_q]));  // qlearning.py:51-66
+    if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.h.gamma, tb.phi[p.phi_row + r.q]), tb.phi[p.phi_row + r.prev_q]));  // qlearning.py:51-66
     update_q(p, Q, V, obs_cell * p.nQ + r.prev_q, action, rew, r.cell * p.nQ + r.q, term_arg, acc);
   }
 }
@@ -474,7 +486,7 @@ __device__ __forceinline__ void reset_slot(const KP& p, const Tab& tb, long long
   s.time = 0;
   s.rm = 0;  // the initial RM state has index 0 (reward_machine.py:32-36)
   s.flags = RLRM_FLAG_ACTIVE | RLRM_FLAG_FIRST;
-  if (p.decay_on_reset) eps = fmax(p.eps_end, __dmul_rn(eps, p.eps_decay));  // learn_done_episode (qlearning.py:153-155)
+  if (p.decay_on_reset) eps = fmax(p.h.eps_end, __dmul_rn(eps, p.h.eps_decay));  // learn_done_episode (qlearning.py:153-155)
 }
 
 __device__ __forceinline__ size_t table_base(const KP& p, long long i, int a) {
@@ -496,6 +508,12 @@ __device__ __forceinline__ void agent_view(const KP& p_in, KP& p, Tab& tb, int a
   tb.rcf += (size_t)a * p_in.nd;
   tb.qrm_states += (size_t)a * p_in.nQ;
   tb.phi += (size_t)a * 2 * p_in.nQ;
+}
+// Sweep handles: the learner settings of instance i's group replace the uniform ones in a copy `p` of the parameter block (one
+// 64-byte load at kernel entry). `i` must be an instance of the launch. Kernels instantiated with SWEEP = false never call it,
+// so their parameter block stays in the constant bank; the unfused entry points call it when sw.hyp is set.
+__device__ __forceinline__ void apply_sweep(KP& p, const Sweep& sw, long long i) {
+  p.h = sw.hyp[((long long)p.instance_offset + i) / sw.group];
 }
 __device__ __forceinline__ Acc make_acc(const KP& p, const DState& st, size_t base) {
   Acc acc = {nullptr, nullptr, nullptr, false, nullptr};

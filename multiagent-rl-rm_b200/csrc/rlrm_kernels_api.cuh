@@ -5,13 +5,14 @@
 // ------------------------------------------------------------------------------------------------
 // unfused kernels (the reference's call-by-call API; also the parity path with injected draws)
 // ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) reset_kernel(KP p, DState st, const unsigned char* mask, unsigned long long t) {
+__global__ void __launch_bounds__(256) reset_kernel(KP p, DState st, const unsigned char* mask, unsigned long long t, Sweep sw) {
   Tab tb = stage_tables(p);
   const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= st.N * p.A) return;
   const long long i = k / p.A;
   const int a = (int)(k - i * p.A);
   if (mask && !mask[i]) return;
+  if (sw.hyp) apply_sweep(p, sw, i);  // the epsilon decay of the instance's group
   Slot s;
   double eps = st.epsilon[k];
   reset_slot(p, tb, i, a, t, s, eps);
@@ -223,7 +224,7 @@ __global__ void __launch_bounds__(256) rm_step_kernel(KP p_in, int agent, long l
 
 template <int ALGO, bool PA, typename T>
 __global__ void __launch_bounds__(256) update_kernel(KP p_in, DState st, const unsigned short* obs_cell, const unsigned char* actions,
-                                                    const unsigned char* term_arg, DOut o) {
+                                                    const unsigned char* term_arg, DOut o, Sweep sw) {
   KP p = p_in;
   Tab tb = stage_tables(p_in);
   const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -231,6 +232,7 @@ __global__ void __launch_bounds__(256) update_kernel(KP p_in, DState st, const u
   const long long i = k / p.A;
   const int a = (int)(k - i * p.A);
   if (PA) agent_view(p_in, p, tb, a);
+  if (sw.hyp) apply_sweep(p, sw, i);
   // the record and the arguments are caller memory: clamp every index that addresses a table
   const unsigned cmax = (unsigned)p.ncell - 1u, qmax = (unsigned)p.nQ - 1u;
   Rec r;
@@ -286,9 +288,9 @@ __device__ __forceinline__ void qlambda_sweep(const KP& p, T* Q, T* E, unsigned 
   const T qsa = Q[s * 4 + a];
   __syncthreads();
   const double best = terminated ? 0.0 : (double)row_max(nrow);
-  const T td = R::sub(R::cvt(__dadd_rn(reward, __dmul_rn(p.gamma, best))), qsa);
+  const T td = R::sub(R::cvt(__dadd_rn(reward, __dmul_rn(p.h.gamma, best))), qsa);
   const T c = R::mul(R::lr(p), td);
-  const bool lr_none = p.lr < 0.0;  // lr = 1 / visits[s, a] (np.float64): the add happens in float64 (qlearning_lambda.py:44-49, 63)
+  const bool lr_none = p.h.lr < 0.0;  // lr = 1 / visits[s, a] (np.float64): the add happens in float64 (qlearning_lambda.py:44-49, 63)
   const double c64 = lr_none ? __dmul_rn(__ddiv_rn(1.0, (double)(visits_now ? visits_now : 1u)), (double)td) : 0.0;
   const unsigned hot = s * 4 + a;
   row_t* Q4 = reinterpret_cast<row_t*>(Q);
@@ -298,7 +300,7 @@ __device__ __forceinline__ void qlambda_sweep(const KP& p, T* Q, T* E, unsigned 
 
 template <typename T>
 __global__ void __launch_bounds__(256) update_qlambda_kernel(KP p_in, DState st, const unsigned short* obs_cell,
-                                                            const unsigned char* actions, const unsigned char* term_arg, DOut o) {
+                                                            const unsigned char* actions, const unsigned char* term_arg, DOut o, Sweep sw) {
   KP p = p_in;
   const long long k = blockIdx.x;
   const long long i = k / p.A;
@@ -308,6 +310,7 @@ __global__ void __launch_bounds__(256) update_qlambda_kernel(KP p_in, DState st,
     p.nQ = p_in.a_nQ[a];
     p.S4 = (long long)p_in.ncell * p.nQ * 4;
   }
+  if (sw.hyp) apply_sweep(p, sw, i);
   // caller memory: clamp what indexes a table
   const unsigned cmax = (unsigned)p.ncell - 1u, qmax = (unsigned)p.nQ - 1u;
   const unsigned s_idx = min((unsigned)obs_cell[k], cmax) * p.nQ + min((unsigned)o.prev_q[k], qmax);
@@ -336,15 +339,17 @@ struct SelArgs {  // the input half of rlrm_select_req_t, passed by value (read 
 };
 template <typename T>
 __global__ void __launch_bounds__(256) update_list_kernel(KP p, DState st, long long slot, int n, const rlrm_experience_t* ex,
-                                                         rlrm_select_req_t* sel, SelArgs sa) {
+                                                         rlrm_select_req_t* sel, SelArgs sa, Sweep sw) {
   const long long i = slot / p.A;
   const int a = (int)(slot - i * p.A);
+  KP pl = p;  // the slot's learner settings (a sweep handle's group); p itself stays in the constant bank
+  if (sw.hyp) apply_sweep(pl, sw, i);
   const size_t base = table_base(p, i, a);
   const unsigned rows = (unsigned)p.ncell * (unsigned)(p.per_agent ? p.a_nQ[a] : p.nQ);
   T* Q = tab<T>(st.q) + base;
   unsigned* V = st.visits ? st.visits + base : nullptr;
   if (p.algo == RLRM_ALGO_QLAMBDA) {
-    KP pa = p;
+    KP pa = pl;
     pa.S4 = (long long)rows * 4;
     T* E = tab<T>(st.e) + base;
     for (int j = 0; j < n; j++) {
@@ -362,7 +367,7 @@ __global__ void __launch_bounds__(256) update_list_kernel(KP p, DState st, long 
   } else if (threadIdx.x == 0) {
     const Acc none = {nullptr, nullptr, nullptr, false, nullptr};
     for (int j = 0; j < n; j++)
-      update_q<T>(p, Q, V, min(ex[j].s, rows - 1u), min((int)ex[j].action, RLRM_N_ACTIONS - 1), ex[j].reward, min(ex[j].sn, rows - 1u),
+      update_q<T>(pl, Q, V, min(ex[j].s, rows - 1u), min((int)ex[j].action, RLRM_N_ACTIONS - 1), ex[j].reward, min(ex[j].sn, rows - 1u),
                   ex[j].terminated != 0, none);
   }
   // rlrm_update_list_select: the next selection on the updated table (thread 0 is also the thread that wrote the QL / QRM

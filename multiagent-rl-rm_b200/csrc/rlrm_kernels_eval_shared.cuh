@@ -445,8 +445,8 @@ __global__ void __launch_bounds__(SHARED_BLOCK, 1) shared_train_cluster_kernel(K
           const float cur = CL_ROW(Qs, Rs, 4)[action];
           const float mx = *CL_ROW(s_rmax, Rsn, 1);
           const float mf = __fmul_rn(terminated ? 0.0f : 1.0f, mx);
-          const float inner = __fadd_rn(__double2float_rn(rew), __fmul_rn(p.gamma_f, mf));
-          const float out = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur), __fmul_rn(p.lr_f, inner));
+          const float inner = __fadd_rn(__double2float_rn(rew), __fmul_rn(p.h.gamma_f, mf));
+          const float out = __fadd_rn(__fmul_rn(p.h.one_minus_lr_f, cur), __fmul_rn(p.h.lr_f, inner));
           const unsigned long long v = (unsigned long long)__float2ll_rn(__fmul_rn(out, 1048576.0f));
           unsigned* wsum = reinterpret_cast<unsigned*>(CL_ROW(s_sum, Rs, 4) + action);
           const unsigned lo = (unsigned)v, hi = (unsigned)(v >> 32);
@@ -465,14 +465,14 @@ __global__ void __launch_bounds__(SHARED_BLOCK, 1) shared_train_cluster_kernel(K
             const double ru = d == RLRM_NO_TRANSITION ? 0.0 : tb.rcf[u * (p.nEv + 1) + col];
             const bool done = r.env_term || (p.rm_final >= 0 && (int)un == p.rm_final);
             double rew = __dadd_rn(r.renv, ru);
-            if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.gamma, tb.phi[un]), tb.phi[u]));
+            if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.h.gamma, tb.phi[un]), tb.phi[u]));
             propose(R0 + r.prev_cell * p.nQ + u, rew, R0 + r.cell * p.nQ + un, done);
           }
         } else {
           const unsigned obs = (p.driver == RLRM_DRIVER_FROZEN_LAKE_MAIN && first) ? r.cell : before;
           const bool term_arg = p.driver == RLRM_DRIVER_FROZEN_LAKE_MAIN ? (r.term || r.trunc) : r.term;
           double rew = r.reward;
-          if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.gamma, tb.phi[p.phi_row + r.q]), tb.phi[p.phi_row + r.prev_q]));
+          if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.h.gamma, tb.phi[p.phi_row + r.q]), tb.phi[p.phi_row + r.prev_q]));
           propose(R0 + obs * p.nQ + r.prev_q, rew, R0 + r.cell * p.nQ + r.q, term_arg);
         }
         term = r.term;

@@ -5,14 +5,16 @@
 
 // PA = agents carry different reward machines: the warp's agent gets its own view of the parameters (a private copy); with
 // PA = false the parameter block stays in the constant bank
-template <int ENV, typename T, bool PA>
+// SWEEP: the block's instance takes its group's learner settings
+template <int ENV, typename T, bool PA, bool SWEEP>
 __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, unsigned long long t0, int n_iters, int learn,
-                                                           unsigned* trace, double* reward_out) {
+                                                           unsigned* trace, double* reward_out, Sweep sw) {
   typedef RT<T> R;
   typedef typename R::row_t row_t;
-  KP p_view;
+  KP p_view, p_sw;  // p_sw: a sweep handle's learner settings, read only where they are used (ph; see train_ql_fast_kernel)
   if (PA) p_view = p_in;
   const KP& p = PA ? p_view : p_in;
+  const KP& ph = SWEEP ? p_sw : p;
   Tab tb = stage_tables(p_in);
   __shared__ int sh_term[RLRM_MAX_AGENTS], sh_trunc[RLRM_MAX_AGENTS];
   const long long i = blockIdx.x;
@@ -20,6 +22,10 @@ __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, 
   const int lane = threadIdx.x & 31;
   const long long k = i * p_in.A + a;
   if (PA) agent_view(p_in, p_view, tb, a);  // this warp's agent has its own machine: nQ, final state, table size
+  if (SWEEP) {
+    p_sw = p;
+    apply_sweep(p_sw, sw, i);
+  }
   Slot s = unpack_slot(st.slot[k]);
   double eps = st.epsilon[k];
   double ep_ret = st.ep_return ? st.ep_return[k] : 0.0;
@@ -56,12 +62,12 @@ __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, 
       const T qsa = Q[sidx * 4 + action];
       __syncwarp();
       const double best = term_arg ? 0.0 : (double)row_max(nrow);
-      const T td = R::sub(R::cvt(__dadd_rn(r.reward, __dmul_rn(p.gamma, best))), qsa);
-      const T c = R::mul(R::lr(p), td);
+      const T td = R::sub(R::cvt(__dadd_rn(r.reward, __dmul_rn(ph.h.gamma, best))), qsa);
+      const T c = R::mul(R::lr(ph), td);
       const unsigned hot = sidx * 4 + action;
       // learning_rate=None: lr = 1 / visits[s, a] is an np.float64, so lr * td and (lr * td) * e_table are float64 and the
       // in-place add happens in float64 before the cast back to float32 (qlearning_lambda.py:44-49, 63)
-      const bool lr_none = p.lr < 0.0;
+      const bool lr_none = ph.h.lr < 0.0;
       unsigned vis = 0;
       if (V) {
         vis = V[hot] + 1;
@@ -71,7 +77,7 @@ __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, 
       const double c64 = lr_none ? __dmul_rn(__ddiv_rn(1.0, (double)vis), (double)td) : 0.0;
       row_t* Q4 = reinterpret_cast<row_t*>(Q);
       row_t* E4 = reinterpret_cast<row_t*>(E);
-      for (long long j = lane; j < p.S4 / 4; j += 32) sweep_row<T>(p, Q4, E4, j, hot, c, c64, lr_none, term_arg);
+      for (long long j = lane; j < p.S4 / 4; j += 32) sweep_row<T>(ph, Q4, E4, j, hot, c, c64, lr_none, term_arg);
       __syncwarp();
     }
     ep_ret = __dadd_rn(ep_ret, r.reward);
@@ -100,7 +106,7 @@ __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, 
       last_length = s.time;
       had_episode = true;
       ep_ret = 0.0;
-      reset_slot(p, tb, i, a, t + 1, s, eps);
+      reset_slot(ph, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
       // reset_e_table (ma_office.py:101-102)
       row_t* E4 = reinterpret_cast<row_t*>(E);
@@ -171,15 +177,16 @@ __device__ __forceinline__ void trace_flush(T* Q, const TraceList<T>& L, unsigne
                                // config 4's scenario with 1 / 2 / 4 agents): 1 agent 32 -> 8 lanes 1.82e9 -> 3.81e9, 2 agents 16 -> 8 lanes 3.05e9 -> 3.95e9;
                                // 4 lanes halve the rate everywhere (the visited entry's lookup needs a second round, a sweep waits for the longest of 8 lists)
 #endif
-template <int ENV, typename T, bool PA>
+template <int ENV, typename T, bool PA, bool SWEEP>
 __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in, DState st, unsigned long long t0, int n_iters, int learn,
-                                                                        unsigned* trace, double* reward_out) {
+                                                                        unsigned* trace, double* reward_out, Sweep sw) {
   typedef RT<T> R;
   typedef typename R::row_t row_t;
   typedef typename R::pair_t pair_t;
-  KP p_view;
+  KP p_view, p_sw;  // p_sw: a sweep handle's learner settings, read only where they are used (ph; see train_ql_fast_kernel)
   if (PA) p_view = p_in;
   const KP& p = PA ? p_view : p_in;
+  const KP& ph = SWEEP ? p_sw : p;
   Tab tb = stage_tables(p_in);
   // lanes per agent LG (p.qls_lg: 4 .. 32 / G) -> lanes per instance LI = LG * G -> 32 / LI instances per warp
   const unsigned FULL = 0xFFFFFFFFu;
@@ -197,6 +204,10 @@ __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in
   const unsigned inst_mask = (LI == 32 ? FULL : ((1u << LI) - 1u)) << (lane & ~(LI - 1));  // the lanes of this lane's instance
   const long long k = i * p_in.A + (valid ? a : 0);
   if (PA) agent_view(p_in, p_view, tb, valid ? a : 0);  // this lane group's agent has its own machine
+  if (SWEEP) {
+    p_sw = p;
+    apply_sweep(p_sw, sw, i);
+  }  // i is clamped to the launch's instances
   Slot s = {0, 0, 0, 0, 0};
   double eps = 0.0, ep_ret = 0.0, return_sum = 0.0;
   T* Q = tab<T>(st.q) + table_base(p_in, i, valid ? a : 0);
@@ -275,9 +286,9 @@ __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in
       row_t nrow;
       nrow.x = n0; nrow.y = n1; nrow.z = n2; nrow.w = n3;
       const double best = term_arg ? 0.0 : (double)row_max(nrow);
-      const T td = R::sub(R::cvt(__dadd_rn(r.reward, __dmul_rn(p.gamma, best))), qsa);
-      const T c = R::mul(R::lr(p), td);
-      const bool lr_none = p.lr < 0.0;  // lr = 1 / visits: float64 arithmetic, see train_qlambda_kernel
+      const T td = R::sub(R::cvt(__dadd_rn(r.reward, __dmul_rn(ph.h.gamma, best))), qsa);
+      const T c = R::mul(R::lr(ph), td);
+      const bool lr_none = ph.h.lr < 0.0;  // lr = 1 / visits: float64 arithmetic, see train_qlambda_kernel
       unsigned vis = 0;
       if (V && valid) {
         vis = V[hot] + 1;
@@ -289,7 +300,7 @@ __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in
         pair_t eq = L.eq[j];
         if (j + 1 == hotpos) eq.x = (T)1;  // replacing trace on the visited entry
         eq.y = lr_none ? R::cvt(__dadd_rn((double)eq.y, __dmul_rn(c64, (double)eq.x))) : R::add(eq.y, R::mul(c, eq.x));
-        eq.x = term_arg ? (T)0 : R::mul(eq.x, R::decay(p));
+        eq.x = term_arg ? (T)0 : R::mul(eq.x, R::decay(ph));
         L.eq[j] = eq;
       }
       work += len;
@@ -297,7 +308,7 @@ __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in
         if (gl == 0) {
           L.idx[len] = (unsigned short)hot;
           const T q_new = lr_none ? R::cvt(__dadd_rn((double)qsa, __dmul_rn(c64, 1.0))) : R::add(qsa, R::mul(c, (T)1));
-          L.eq[len] = R::make_pair(term_arg ? (T)0 : R::mul((T)1, R::decay(p)), q_new);
+          L.eq[len] = R::make_pair(term_arg ? (T)0 : R::mul((T)1, R::decay(ph)), q_new);
           L.pos[hot] = (unsigned short)(len + 1);
         }
         len++;
@@ -322,7 +333,7 @@ __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in
       last_length = s.time;
       had_episode = true;
       ep_ret = 0.0;
-      reset_slot(p, tb, i, a, t + 1, s, eps);
+      reset_slot(ph, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
       wipe = true;  // reset_e_table (ma_office.py:101-102)
     }

@@ -21,13 +21,19 @@
 #endif
 
 // T = table arithmetic type (float: float32 tables; double: the reference's native float64 tables, see RT<T>)
-template <int ENV, int ALGO, bool PA, typename T>
+// SWEEP: the handle carries per-group learner settings (rlrm_set_sweep); every fused kernel takes the flag the same way
+template <int ENV, int ALGO, bool PA, typename T, bool SWEEP>
 __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_kernel(KP p_in, DState st, unsigned long long t0, int n_iters, int learn,
-                                                           unsigned* trace, double* reward_out) {
+                                                           unsigned* trace, double* reward_out, Sweep sw) {
   typedef RT<T> R;
   typedef typename R::row_t row_t;
   KP p = p_in;
   Tab tb = stage_tables(p_in);
+  // SWEEP: the instance's learner settings go into a separate copy read only where they are used (ph). The parameter block
+  // (with PA, the per-agent view) is indexed dynamically (slip outcomes) and would move to local memory as a whole if it were written.
+  KP p_sw;
+  if (SWEEP) p_sw = p;
+  const KP& ph = SWEEP ? p_sw : p;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long i = tid >> p.g_shift;
   const int a = (int)(tid & (p.G - 1));
@@ -51,6 +57,10 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
     if (st.ep_return) ep_ret = st.ep_return[k];
     if (st.stats) return_sum = st.stats[k].return_sum;
     if (PA) agent_view(p_in, p, tb, a);
+    if (SWEEP) {
+      p_sw = p;  // after the per-agent view
+      apply_sweep(p_sw, sw, i);
+    }
     const size_t base = table_base(p_in, i, a);
     Q = tab<T>(st.q) + base;
     V = st.visits ? st.visits + base : nullptr;
@@ -59,7 +69,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
   unsigned long long explore_thr = explore_threshold(eps);
   bool had_episode = false;
   // plain QL with a private table, fixed learning rate and no visit counts: carry the current row across iterations
-  const bool carry = (ALGO == RLRM_ALGO_QL) && !V && !acc.sum && p.lr >= 0.0;
+  const bool carry = (ALGO == RLRM_ALGO_QL) && !V && !acc.sum && ph.h.lr >= 0.0;
   row_t row = R::zero_row();
   unsigned row_idx = 0xFFFFFFFFu;
 
@@ -93,10 +103,10 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
           const T cur = (sidx == row_idx) ? get_component(row, action)
                                                : ((sidx == snidx) ? get_component(nrow, action) : Q[(size_t)sidx * 4 + action]);
           double rew = r.reward;
-          if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.gamma, tb.phi[p.phi_row + r.q]), tb.phi[p.phi_row + r.prev_q]));
+          if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(ph.h.gamma, tb.phi[p.phi_row + r.q]), tb.phi[p.phi_row + r.prev_q]));
           const T mf = R::mul(term_arg ? (T)0 : (T)1, row_max(nrow));
-          const T inner = R::add(R::cvt(rew), R::mul(R::gamma(p), mf));
-          const T out = R::add(R::mul(R::one_minus_lr(p), cur), R::mul(R::lr(p), inner));
+          const T inner = R::add(R::cvt(rew), R::mul(R::gamma(ph), mf));
+          const T out = R::add(R::mul(R::one_minus_lr(ph), cur), R::mul(R::lr(ph), inner));
           if (!R::same_bits(out, cur)) Q[(size_t)sidx * 4 + action] = out;
           if (sidx == row_idx) set_component(row, action, out);
           if (snidx != row_idx) {  // the next state's row becomes the carried one
@@ -105,7 +115,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
             row_idx = snidx;
           }
         } else {
-          agent_update<ALGO, T>(p, tb, Q, V, obs, action, term_arg, r, acc);
+          agent_update<ALGO, T>(ph, tb, Q, V, obs, action, term_arg, r, acc);
         }
       }
       term = r.term;
@@ -129,7 +139,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
       last_length = s.time;
       had_episode = true;
       ep_ret = 0.0;
-      reset_slot(p, tb, i, a, t + 1, s, eps);  // next episode starts with rm_env.reset (frozen_lake_main.py:337)
+      reset_slot(ph, tb, i, a, t + 1, s, eps);  // next episode starts with rm_env.reset (frozen_lake_main.py:337)
       explore_thr = explore_threshold(eps);
     }
   }
@@ -228,9 +238,9 @@ __device__ __forceinline__ float max4(const float* v) { return fmaxf(fmaxf(v[0],
 // registers are short (the 72-register MINB 7 case). The same-cell patches of the block are selects. Every Q store of
 // iteration t precedes the fetch of t+1 in program order: an agent that steps back into the cell it just left must read
 // what it wrote.
-template <int ENV, bool STOCH, bool LEARN, bool TRACE, int MINB>
+template <int ENV, bool STOCH, bool LEARN, bool TRACE, int MINB, bool SWEEP>
 __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DState st, unsigned long long t0, int n_iters,
-                                                                unsigned* trace) {
+                                                                unsigned* trace, Sweep sw) {
   Tab tb = stage_tables(p);
   const unsigned sm = smem_addr();
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -253,6 +263,8 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
   for (int j = 0; j < 16; j++) B[j] = 0.f;
   unsigned w[4] = {0u, 0u, 0u, 0u}, sidx = 0u;  // Philox words and slip threshold index of the coming iteration
   if (valid) {
+    // nothing here indexes the parameter block dynamically: the written settings stay in registers, the rest in the constant bank
+    if (SWEEP) apply_sweep(p, sw, i);
     s = unpack_slot(st.slot[k]);
     eps = st.epsilon[k];
     if (st.ep_return) ep_ret = st.ep_return[k];
@@ -372,8 +384,8 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, MINB) train_qrm4_kernel(KP p, DSt
         const bool done = env_term || ((rec.w >> (6 + u)) & 1u);
         const float mx = sel4(bmax[0], bmax[1], bmax[2], bmax[3], un);
         const float mf = __fmul_rn(done ? 0.0f : 1.0f, mx);
-        const float inner = __fadd_rn(cf[u], __fmul_rn(p.gamma_f, mf));
-        const float nv = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur[u]), __fmul_rn(p.lr_f, inner));
+        const float inner = __fadd_rn(cf[u], __fmul_rn(p.h.gamma_f, mf));
+        const float nv = __fadd_rn(__fmul_rn(p.h.one_minus_lr_f, cur[u]), __fmul_rn(p.h.lr_f, inner));
         if (__float_as_uint(nv) != __float_as_uint(cur[u])) dst[4 * u] = nv;  // a bit-identical value needs no store
         // same cell: the carried block is the one just written
 #pragma unroll
@@ -443,9 +455,15 @@ __device__ __forceinline__ void load_block_n(const float* Q, unsigned cell, floa
   }
 }
 
-template <int ENV, int NQ, bool STOCH, bool LEARN, bool TRACE>
-__global__ void __launch_bounds__(TRAIN_BLOCK, 7) train_qrmn_kernel(KP p, DState st, unsigned long long t0, int n_iters, unsigned* trace) {
+template <int ENV, int NQ, bool STOCH, bool LEARN, bool TRACE, bool SWEEP>
+__global__ void __launch_bounds__(TRAIN_BLOCK, 7) train_qrmn_kernel(KP p, DState st, unsigned long long t0, int n_iters, unsigned* trace,
+                                                                   Sweep sw) {
   Tab tb = stage_tables(p);
+  // SWEEP: the instance's learner settings go into a separate copy read only where they are used (ph). The parameter block
+  // itself is indexed dynamically (slip outcomes) and would move to local memory as a whole if it were written.
+  KP p_sw;
+  if (SWEEP) p_sw = p;
+  const KP& ph = SWEEP ? p_sw : p;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long i = tid >> p.g_shift;
   const int a = (int)(tid & (p.G - 1));
@@ -464,6 +482,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, 7) train_qrmn_kernel(KP p, DState
 #pragma unroll
   for (int j = 0; j < NQ; j++) bmax[j] = 0.f;
   if (valid) {
+    if (SWEEP) apply_sweep(p_sw, sw, i);
     s = unpack_slot(st.slot[k]);
     eps = st.epsilon[k];
     if (st.ep_return) ep_ret = st.ep_return[k];
@@ -506,8 +525,8 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, 7) train_qrmn_kernel(KP p, DState
           const bool done = r.env_term || (p.rm_final >= 0 && (int)un == p.rm_final);
           const float mx = sel_state<NQ>(bmax, 1, un);
           const float mf = __fmul_rn(done ? 0.0f : 1.0f, mx);
-          const float inner = __fadd_rn(__double2float_rn(__dadd_rn(r.renv, ru)), __fmul_rn(p.gamma_f, mf));
-          const float nv = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur[u]), __fmul_rn(p.lr_f, inner));
+          const float inner = __fadd_rn(__double2float_rn(__dadd_rn(r.renv, ru)), __fmul_rn(ph.h.gamma_f, mf));
+          const float nv = __fadd_rn(__fmul_rn(ph.h.one_minus_lr_f, cur[u]), __fmul_rn(ph.h.lr_f, inner));
           if (__float_as_uint(nv) != __float_as_uint(cur[u])) dst[4 * u] = nv;  // a bit-identical value needs no store
           if (!moved) {  // same cell: the carried block is the one just written
 #pragma unroll
@@ -536,7 +555,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, 7) train_qrmn_kernel(KP p, DState
       last_length = s.time;
       had_episode = true;
       ep_ret = 0.0;
-      reset_slot<false>(p, tb, i, a, t + 1, s, eps);
+      reset_slot<false>(ph, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
       load_block_n<NQ>(Q, s.cell, B, bmax);
     }
@@ -665,13 +684,18 @@ struct BlkRow<double, CS> {
 
 // T = table type: float, or double for the reference's native float64 tables (a row is then two 16-byte chunks; BASELINE config 3's
 // four-state machine in float64 takes this kernel too: 128 bytes of block per thread)
-template <int ENV, int NU, typename T, bool TMA>
+template <int ENV, int NU, typename T, bool TMA, bool SWEEP>
 __global__ void __launch_bounds__(TRAIN_BLOCK, QRMB_MINB(T)) train_qrm_block_kernel(KP p, DState st, unsigned long long t0, int n_iters, int learn,
-                                                                                unsigned* trace) {
+                                                                                unsigned* trace, Sweep sw) {
   typedef RT<T> R;
   typedef BlkRow<T, TMA ? 1 : TRAIN_BLOCK> BR;
   typedef typename R::row_t row_t;
   Tab tb = stage_tables(p);
+  // SWEEP: the instance's learner settings go into a separate copy read only where they are used (ph). The parameter block
+  // itself is indexed dynamically (slip outcomes) and would move to local memory as a whole if it were written.
+  KP p_sw;
+  if (SWEEP) p_sw = p;
+  const KP& ph = SWEEP ? p_sw : p;
   unsigned char* area = smem_raw + ((p.blob_bytes + 15) & ~15);
   unsigned bar = 0, phase = 0;
   uint4* blk;
@@ -705,6 +729,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QRMB_MINB(T)) train_qrm_block_ker
   unsigned episodes = 0, successes = 0, last_length = 0;
   float last_return = 0.f;
   if (valid) {
+    if (SWEEP) apply_sweep(p_sw, sw, i);
     s = unpack_slot(st.slot[k]);
     eps = st.epsilon[k];
     if (st.ep_return) ep_ret = st.ep_return[k];
@@ -747,10 +772,10 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QRMB_MINB(T)) train_qrm_block_ker
             const double ru = d == RLRM_NO_TRANSITION ? 0.0 : tb.rcf[u * nE1 + col];
             const bool done = r.env_term || (p.rm_final >= 0 && (int)un == p.rm_final);
             double rew = __dadd_rn(r.renv, ru);
-            if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(p.gamma, tb.phi[un]), tb.phi[u]));  // qlearning.py:93-105
+            if (p.use_rsh) rew = __dadd_rn(rew, __dsub_rn(__dmul_rn(ph.h.gamma, tb.phi[un]), tb.phi[u]));  // qlearning.py:93-105
             const T mf = R::mul(done ? (T)0 : (T)1, row_max(BR::load(blk, un)));
-            const T inner = R::add(R::cvt(rew), R::mul(R::gamma(p), mf));
-            const T nv = R::add(R::mul(R::one_minus_lr(p), cur[j]), R::mul(R::lr(p), inner));
+            const T inner = R::add(R::cvt(rew), R::mul(R::gamma(ph), mf));
+            const T nv = R::add(R::mul(R::one_minus_lr(ph), cur[j]), R::mul(R::lr(ph), inner));
             if (!R::same_bits(nv, cur[j])) dst[4 * u] = nv;  // a bit-identical value needs no store
             if (!moved) BR::set(blk, u, action, nv);  // same cell: the shared block is the one just written
           }
@@ -779,7 +804,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QRMB_MINB(T)) train_qrm_block_ker
       had_episode = true;
       ep_ret = 0.0;
       const unsigned old_cell = s.cell;
-      reset_slot(p, tb, i, a, t + 1, s, eps);
+      reset_slot(ph, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
       if (s.cell != old_cell) QRMB_FETCH_BLOCK(Q + (size_t)s.cell * (size_t)(nQ * 4));
     }
@@ -811,10 +836,15 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QRMB_MINB(T)) train_qrm_block_ker
 // agent's current state stays in registers, one 16-byte load of Q[s'] and at most one 4-byte store per step — with the
 // run-time switches (stochastic / learn / trace / per-agent views / random starts / shared accumulators) compiled out.
 // ------------------------------------------------------------------------------------------------
-template <int ENV, bool STOCH, bool LEARN, bool TRACE>
+template <int ENV, bool STOCH, bool LEARN, bool TRACE, bool SWEEP>
 __global__ void __launch_bounds__(TRAIN_BLOCK, QLF_MINB) train_ql_fast_kernel(KP p, DState st, unsigned long long t0, int n_iters,
-                                                                   unsigned* trace) {
+                                                                   unsigned* trace, Sweep sw) {
   Tab tb = stage_tables(p);
+  // SWEEP: the instance's learner settings go into a separate copy read only where they are used (ph). The parameter block
+  // itself is indexed dynamically (slip outcomes) and would move to local memory as a whole if it were written.
+  KP p_sw;
+  if (SWEEP) p_sw = p;
+  const KP& ph = SWEEP ? p_sw : p;
   const long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   const long long i = tid >> p.g_shift;
   const int a = (int)(tid & (p.G - 1));
@@ -830,6 +860,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QLF_MINB) train_ql_fast_kernel(KP
   float4 row = make_float4(0.f, 0.f, 0.f, 0.f);  // Q[row_idx, :], the 1-entry register cache of the table
   unsigned row_idx = 0;
   if (valid) {
+    if (SWEEP) apply_sweep(p_sw, sw, i);
     s = unpack_slot(st.slot[k]);
     eps = st.epsilon[k];
     if (st.ep_return) ep_ret = st.ep_return[k];
@@ -868,8 +899,8 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QLF_MINB) train_ql_fast_kernel(KP
         float cur = (sidx == row_idx) ? row_a : nrow_a;
         if (sidx != row_idx && sidx != snidx) cur = Q[(size_t)sidx * 4 + action];  // only the aliased first iteration gets here
         const float mf = __fmul_rn(term_arg ? 0.0f : 1.0f, row_max(nrow));
-        const float inner = __fadd_rn(__double2float_rn(r.reward), __fmul_rn(p.gamma_f, mf));
-        const float out = __fadd_rn(__fmul_rn(p.one_minus_lr_f, cur), __fmul_rn(p.lr_f, inner));
+        const float inner = __fadd_rn(__double2float_rn(r.reward), __fmul_rn(ph.h.gamma_f, mf));
+        const float out = __fadd_rn(__fmul_rn(ph.h.one_minus_lr_f, cur), __fmul_rn(ph.h.lr_f, inner));
         if (__float_as_uint(out) != __float_as_uint(cur)) Q[(size_t)sidx * 4 + action] = out;
         const bool same = sidx == snidx;  // the updated entry belongs to the row carried into the next iteration
         nrow.x = (same && action == 0) ? out : nrow.x;
@@ -899,7 +930,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, QLF_MINB) train_ql_fast_kernel(KP
       last_length = s.time;
       had_episode = true;
       ep_ret = 0.0;
-      reset_slot<false>(p, tb, i, a, t + 1, s, eps);
+      reset_slot<false>(ph, tb, i, a, t + 1, s, eps);
       explore_thr = explore_threshold(eps);
       row_idx = s.cell * p.nQ + s.rm;
       row = *reinterpret_cast<const float4*>(Q + (size_t)row_idx * 4);

@@ -8,7 +8,7 @@ agent with its own Reward-Machine state, learner table and epsilon. torch is use
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Optional
+from typing import Dict, List, Optional
 
 import numpy as np
 import torch
@@ -31,16 +31,54 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else t.data_ptr()
 
 
+SWEEP_KEYS = ("learning_rate", "gamma", "lambd", "epsilon_start", "epsilon_end", "epsilon_decay")
+
+
+def sweep_settings(scenario, sweep) -> List[dict]:
+    """The settings of a hyper-parameter sweep with every key of SWEEP_KEYS present: keys a setting leaves out come from
+    `scenario`. learning_rate None is 1 / visits, as in the scenario. Raises ValueError on anything malformed."""
+    if isinstance(sweep, dict) or not hasattr(sweep, "__len__") or len(sweep) == 0:
+        raise ValueError("sweep must be a non-empty list of dicts")
+    if scenario.shared_q:
+        raise ValueError("a sweep needs per-instance tables: the instances of a shared table share one learner")
+    out = []
+    for j, setting in enumerate(sweep):
+        if not isinstance(setting, dict):
+            raise ValueError(f"sweep[{j}] is not a dict")
+        unknown = set(setting) - set(SWEEP_KEYS)
+        if unknown:
+            raise ValueError(f"sweep[{j}] has unknown keys {sorted(unknown)}; allowed: {SWEEP_KEYS}")
+        s = {k: setting.get(k, getattr(scenario, k)) for k in SWEEP_KEYS}
+        for k in SWEEP_KEYS:
+            if s[k] is None and k == "learning_rate":
+                continue
+            if isinstance(s[k], bool) or not isinstance(s[k], (int, float)):
+                raise ValueError(f"sweep[{j}][{k!r}] must be a number")
+            s[k] = float(s[k])
+        if s["learning_rate"] is not None and s["learning_rate"] < 0:
+            raise ValueError(f"sweep[{j}]: learning_rate must be >= 0 or None")
+        if scenario.use_rsh and s["gamma"] != float(scenario.gamma):
+            # the shaping potentials are built from the scenario's gamma (RewardMachine.add_reward_shaping)
+            raise ValueError(f"sweep[{j}]: reward shaping takes the scenario's gamma; a setting cannot change it")
+        out.append(s)
+    return out
+
+
 class Engine:
     def __init__(self, compiled: Compiled, n_instances: int, device="cuda:0", track_visits: bool = False,
-                 with_stats: bool = True, qlambda_sparse: bool = False, host_control: bool = False):
+                 with_stats: bool = True, qlambda_sparse: bool = False, host_control: bool = False, sweep=None,
+                 sweep_group: Optional[int] = None):
         """host_control: keep the small per-slot control state (slot words, epsilon, running return) in page-locked HOST
         memory instead of device memory. Page-locked memory is device-accessible under unified addressing, so the kernels
         read / write it in place and a host driver (the one-instance reference-shaped classes in envs.py) touches it through
         numpy views without any copy. Meant for small N; large batches keep it in HBM.
         qlambda_sparse: Q(lambda) only — keep the traces as per-agent lists of live entries (sparse-exact, see
         include/rlrm_b200.h) instead of the dense e table. Same results bit for bit, far less memory traffic; the fused
-        `train` path only (the call-by-call `update` needs the dense table). Call `sync_tables()` before reading `q`."""
+        `train` path only (the call-by-call `update` needs the dense table). Call `sync_tables()` before reading `q`.
+        sweep: a hyper-parameter sweep, a list of dicts with keys among SWEEP_KEYS (missing keys come from the scenario).
+        Setting g applies to the sweep_group instances with global ids [g * sweep_group, (g + 1) * sweep_group), global id =
+        compiled instance_offset + local index; sweep_group defaults to n_instances // len(sweep), which must then divide
+        evenly. Every instance behaves bit for bit as in an engine built with its setting (rlrm_set_sweep)."""
         self.L = load()
         if not torch.cuda.is_available():
             raise RuntimeError("multiagent-rl-rm_b200 needs a CUDA device (no CPU fallback)")
@@ -48,12 +86,28 @@ class Engine:
         self.cfg = compiled.config
         self.device = torch.device(device)
         self.N, self.A, self.S = int(n_instances), compiled.n_agents, compiled.state_space
+        self.sweep = self.sweep_group = None
+        if sweep is not None:
+            self.sweep = sweep_settings(compiled.scenario, sweep)
+            if sweep_group is None:
+                if self.N % len(self.sweep):
+                    raise ValueError("n_instances must be a multiple of len(sweep) (or pass sweep_group)")
+                sweep_group = self.N // len(self.sweep)
+            self.sweep_group = int(sweep_group)
+            if self.sweep_group <= 0:
+                raise ValueError("sweep_group must be positive")
+            if int(self.cfg.instance_offset) + self.N > len(self.sweep) * self.sweep_group:
+                raise ValueError("the sweep's settings do not cover every instance of this engine")
         dev_index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         self._dev_index = dev_index
         self._tables = compiled.tables_struct()
         h = C.c_void_p()
         check(self.L.rlrm_create(C.byref(self.cfg), C.byref(self._tables), dev_index, C.byref(h)))
         self.h = h
+        if self.sweep is not None:
+            sets = (abi.Hyper * len(self.sweep))(*[abi.Hyper(-1.0 if s["learning_rate"] is None else s["learning_rate"], s["gamma"],
+                                                             s["lambd"], s["epsilon_end"], s["epsilon_decay"]) for s in self.sweep])
+            check(self.L.rlrm_set_sweep(self.h, sets, len(self.sweep), self.sweep_group))
         n_slots = self.N * self.A
         n_tab = self.A if self.cfg.shared_q else n_slots
         tab_shape = (n_tab, self.S, 4)
@@ -81,7 +135,12 @@ class Engine:
             self.tr_eq = torch.zeros((n_slots, self.tr_cap, 2), dtype=self.table_dtype, device=d)  # (trace, q value) pairs
             self.tr_len = torch.zeros(n_slots, dtype=torch.int32, device=d)
             self.tr_work = torch.zeros(n_slots, dtype=torch.int64, device=d)
-        need_visits = track_visits or self.cfg.learning_rate < 0
+        if self.sweep is not None:  # epsilon starts per setting; the kernels carry it per slot from here on
+            g = (int(self.cfg.instance_offset) + torch.arange(self.N)) // self.sweep_group
+            eps0 = torch.tensor([s["epsilon_start"] for s in self.sweep], dtype=torch.float64)[g].repeat_interleave(self.A)
+            self.epsilon.copy_(eps0)
+        lr_none = any(s["learning_rate"] is None for s in self.sweep) if self.sweep is not None else self.cfg.learning_rate < 0
+        need_visits = track_visits or lr_none
         self.visits = torch.zeros(tab_shape, dtype=torch.int32, device=d) if need_visits else None
         self.ep_return = pin(torch.zeros(n_slots, dtype=torch.float64, device=cd))
         self.stats = torch.zeros((n_slots, 32), dtype=torch.uint8, device=d) if with_stats else None
@@ -336,6 +395,29 @@ class Engine:
     def stats_numpy(self):
         return self.stats.cpu().numpy().view(STATS_DTYPE).reshape(-1)
 
+    def group_stats(self) -> Dict[str, torch.Tensor]:
+        """Per-setting totals of the finished episodes' statistics, reduced on the device: tensors [len(sweep)] (a uniform
+        engine is one group) of `episodes`, `successes`, `active_steps` (int64) and `return_sum` (float64). Settings with no
+        instance on this engine (a shard of a sweep) read zero. One learning curve per setting is a series of these."""
+        H, k = (len(self.sweep), self.sweep_group) if self.sweep is not None else (1, self.N)
+        off = int(self.cfg.instance_offset) if self.sweep is not None else 0
+        b = self.stats
+        u32 = b.view(torch.int32).to(torch.int64) & 0xFFFFFFFF
+        fields = {"episodes": u32[:, 2], "successes": u32[:, 3], "active_steps": b.view(torch.int64)[:, 0],
+                  "return_sum": b.view(torch.float64)[:, 2]}
+        lead = off % k  # the engine's instances cover groups g0 .. g0 + m - 1, the first and last possibly in part
+        g0 = off // k
+        m = (lead + self.N + k - 1) // k
+        out = {}
+        for name, v in fields.items():
+            per_inst = v.view(self.N, self.A).sum(dim=1)
+            padded = torch.zeros(m * k, dtype=per_inst.dtype, device=per_inst.device)
+            padded[lead:lead + self.N] = per_inst
+            tot = torch.zeros(H, dtype=per_inst.dtype, device=per_inst.device)
+            tot[g0:g0 + m] = padded.view(m, k).sum(dim=1)
+            out[name] = tot
+        return out
+
     def total_active_steps(self) -> int:
         """Active agent-steps so far = env.agent_steps of every finished episode (stats.active_steps) + the running
         episodes' agent_steps (slot words), reduced on the device."""
@@ -352,12 +434,15 @@ class Engine:
         iteration counter (the Philox counter word). The reference only pickles learner objects (office_main.py:1611-1613,
         1922-1925; see learners.QLearning.__getstate__ for that format); a batch of instances resumes from this instead."""
         out = {k: getattr(self, k).cpu() for k in self._STATE_TENSORS if getattr(self, k) is not None}
-        out.update({"t": int(self.t), "n_instances": self.N, "n_agents": self.A, "state_space": self.S, "sparse": self.sparse})
+        out.update({"t": int(self.t), "n_instances": self.N, "n_agents": self.A, "state_space": self.S, "sparse": self.sparse,
+                    "sweep": None if self.sweep is None else [dict(s) for s in self.sweep], "sweep_group": self.sweep_group})
         return out
 
     def load_state_dict(self, state: Dict[str, object]) -> None:
         if (state["n_instances"], state["n_agents"], state["state_space"], state["sparse"]) != (self.N, self.A, self.S, self.sparse):
             raise ValueError("checkpoint was taken from a differently shaped engine")
+        if (state.get("sweep"), state.get("sweep_group")) != (self.sweep, self.sweep_group):
+            raise ValueError("checkpoint was taken from an engine with a different hyper-parameter sweep")
         for k in self._STATE_TENSORS:
             mine = getattr(self, k)
             if (mine is None) != (k not in state):
