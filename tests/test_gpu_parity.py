@@ -151,6 +151,7 @@ def test_generic_kernel_equals_specialised(name, cuda_device):
     more states / permuted state order / shaping / random starts) — and both with the oracle."""
     import multiagent_rlrm_b200 as P
     import oracle as O
+    from test_fuzz_kernels_gpu import launched_train_kernels
 
     if name == "fl_shaping_qrm":
         sc, n, t = _shaped_qrm(), 400, 1500
@@ -166,7 +167,14 @@ def test_generic_kernel_equals_specialised(name, cuda_device):
     c_gen.config.reserved = 1
     a, b = _engine(c_fast, n), _engine(c_gen, n)
     a.reset(); b.reset()
-    ta, tb = a.train(t, trace=True), b.train(t, trace=True)
+    out = {}
+    ka = launched_train_kernels(lambda: out.update(a=a.train(t, trace=True)))
+    kb = launched_train_kernels(lambda: out.update(b=b.train(t, trace=True)))
+    # the comparison means something only if the two engines ran different kernels. The helper relies on CUPTI's kernel records,
+    # which torch.profiler drops in processes that have run for a minute or more (see launched_train_kernels): this file runs
+    # early enough in the suite, and a dropout fails loudly instead of passing
+    assert [k.family for k in kb] == ["train_kernel"] and len(ka) == 1 and ka[0].family != "train_kernel", (ka, kb)
+    ta, tb = out["a"], out["b"]
     assert np.array_equal(ta.cpu().numpy(), tb.cpu().numpy())
     assert np.array_equal(a.q.cpu().numpy(), b.q.cpu().numpy())
     assert np.array_equal(a.slot.cpu().numpy(), b.slot.cpu().numpy())

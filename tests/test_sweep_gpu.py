@@ -183,6 +183,8 @@ def test_degenerate_sweep_equals_uniform_engine(name, cuda_device):
 @pytest.mark.parametrize("name", ["qrm4_minb7", "ql_fast", "qrmn_3", "qrmn_5", "qrm_block_f32", "qrm_block_f64", "qrm_block_f32_cpasync",
                                   "qrm_block_f64_cpasync", "shaping_qrm"])
 def test_forced_generic_equals_fast_path_under_a_sweep(name, cuda_device):
+    # that these two engines run different kernels is checked by test_forced_generic_sweep_engines_run_different_kernels
+    # (tests/test_fuzz_kernels_gpu.py), early in the suite, where the profiler still records kernels
     sc, sets, k, iters, kw = _case(name)
     n = len(sets) * k
     fast, gen = _engine(sc, n, sweep=sets, **kw), _engine(sc, n, reserved=1, sweep=sets, **kw)
