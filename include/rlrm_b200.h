@@ -343,6 +343,8 @@ int rlrm_update(rlrm_handle_t* h, const rlrm_state_t* st, const uint16_t* obs_ce
  * cooperative launch (tables and proposal accumulators in shared memory, one grid barrier per iteration; tables too large for
  * one SM's 227 KB are partitioned over the distributed shared memory of a thread-block cluster of 2 / 4 / 8 blocks); with a
  * trace buffer, learn = 0 or tables beyond 8 x 227 KB it falls back to two launches per iteration.
+ * Visit counts (state.visits) of a shared table are shared too: each entry counts every proposal made to it, by all
+ * instances, in every iteration.
  * Inter-GPU merging (every K iterations) is the caller's step: average the replicas of `q` (dist.merge_replicas gathers
  * them over NCCL and sums in rank order, so the result does not depend on the collective's reduction order). */
 

@@ -408,7 +408,10 @@ __device__ __forceinline__ void update_q(const KP& p, T* Q, unsigned* V, unsigne
     const double lr = __ddiv_rn(1.0, (double)v);
     out = R::cvt(__dadd_rn(__dmul_rn(__dsub_rn(1.0, lr), (double)cur), __dmul_rn(lr, (double)inner)));
   } else {
-    if (V) V[s * 4 + a] += 1;
+    if (V) {  // a shared table's counts are shared by every instance: count each proposal atomically
+      if (acc.sum) atomicAdd(V + s * 4 + a, 1u);
+      else V[s * 4 + a] += 1;
+    }
     out = R::add(R::mul(R::one_minus_lr(p), cur), R::mul(R::lr(p), inner));
   }
   if (sizeof(T) == 4 && acc.sum) {  // shared learner (float32 tables only): propose; apply_shared_kernel turns the proposals of this iteration into their mean
