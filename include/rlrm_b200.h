@@ -267,6 +267,27 @@ typedef struct rlrm_hyper {
 } rlrm_hyper_t;
 int rlrm_set_sweep(rlrm_handle_t* h, const rlrm_hyper_t* sets, int32_t n_sets, int64_t group_size);
 
+/* Exploration of the selections rlrm_train, rlrm_iterate, rlrm_select_action and rlrm_update_list_select make (best == 0 /
+ * learn != 0; greedy evaluation stays the first argmax). RLRM_EXPLORE_EPSILON_GREEDY (the default) is QLearning.choose_action.
+ * RLRM_EXPLORE_SOFTMAX with temperature tau > 0 and beta = 1.0 / tau (double) selects, for one slot with row Q[0..n-1],
+ * n = cfg.n_actions, Q float or double as the table is:
+ *   1. m = max Q[0..n-1]; d_a = ((double)Q[a] - (double)m) * beta; w_a = E(d_a), so d_a <= 0 and E(0) = 1.0;
+ *   2. C_j = C_{j-1} + w_j in action order (C_0 = w_0), total = C_{n-1};
+ *   3. T_j = (uint64_t)ceil(C_j / total * 2^32) for j < n - 1; action = #{ j < n - 1 : w1 >= T_j }
+ * with every operation a round-to-nearest double operation (no contraction) and w1 the second word of the iteration's Philox
+ * draw (rlrm_select_action's draws[4k + 1]; w3 keeps its slip role, w0 and w2 are unused). E(x), x <= 0, is a fixed operation
+ * sequence (rlrm_exp in the sources): +0 below ln(2^-1075); k = rint(x * log2e); r = fma(-k, ln2_hi, x), r = fma(-k, ln2_lo, r);
+ * the degree-14 Taylor polynomial of exp(r) by Horner's rule with fma; times 2^k built from its bits (2^(k+54), then 2^-54, when
+ * k < -1021).
+ * The constants are in csrc/rlrm_device.cuh and, restated, in tests/softmax_oracle.c. It is within 2 ULP of a correctly rounded exp.
+ * Actions whose weight underflows to 0 are never chosen. epsilon is still carried and decayed per slot, but not read.
+ * RLRM_ERR_ARG for an unknown kind, or a softmax temperature that is not finite, not > 0 or whose reciprocal overflows;
+ * RLRM_ERR_UNSUPPORTED on a shared_q handle. Softmax launches take the generic training kernel (or the Q(lambda) kernels);
+ * kind = RLRM_EXPLORE_EPSILON_GREEDY restores the epsilon-greedy handle exactly, specialised kernels included. */
+#define RLRM_EXPLORE_EPSILON_GREEDY 0
+#define RLRM_EXPLORE_SOFTMAX 1
+int rlrm_set_exploration(rlrm_handle_t* h, int32_t kind, double temperature);
+
 /* RMEnvironmentWrapper.reset (rm_environment_wrapper.py:28-41) -> env.reset (ma_frozen_lake.py:43-94,
  * ma_office.py:77-120): positions, RM state, counters, epsilon decay, Q(lambda) trace wipe.
  * mask: device uint8 [N] selecting instances, or NULL for all. */

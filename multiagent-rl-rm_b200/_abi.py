@@ -18,6 +18,7 @@ ENV_FROZEN_LAKE, ENV_OFFICE_WORLD = 0, 1
 ALGO_QL, ALGO_QRM, ALGO_QLAMBDA = 0, 1, 2
 DRIVER_FROZEN_LAKE_MAIN, DRIVER_OFFICE_MAIN = 0, 1
 TABLE_F32, TABLE_F64 = 0, 1
+EXPLORE_EPSILON_GREEDY, EXPLORE_SOFTMAX = 0, 1
 
 SLOT_CELL_SHIFT, SLOT_STEPS_SHIFT, SLOT_TIME_SHIFT, SLOT_RMSTATE_SHIFT, SLOT_FLAGS_SHIFT = 0, 16, 32, 48, 56
 FLAG_ACTIVE, FLAG_FAIL, FLAG_DONE, FLAG_TRUNC, FLAG_FIRST = 1, 2, 4, 8, 16
@@ -181,6 +182,7 @@ EXPORTED_SYMBOLS = (
     "rlrm_destroy",
     "rlrm_set_learner",
     "rlrm_set_sweep",
+    "rlrm_set_exploration",
     "rlrm_reset",
     "rlrm_reset_at",
     "rlrm_select_action",

@@ -84,6 +84,7 @@ def load():
     L.rlrm_destroy.argtypes = [vp]
     L.rlrm_set_learner.argtypes = [vp, C.c_double, C.c_double, C.c_double]
     L.rlrm_set_sweep.argtypes = [vp, C.POINTER(abi.Hyper), i32, i64]
+    L.rlrm_set_exploration.argtypes = [vp, i32, C.c_double]
     L.rlrm_reset.argtypes = [vp, C.POINTER(abi.State), vp, vp]
     L.rlrm_reset_at.argtypes = [vp, C.POINTER(abi.State), vp, u64, vp]
     L.rlrm_select_action.argtypes = [vp, C.POINTER(abi.State), vp, u64, C.c_int, vp, vp]
@@ -106,7 +107,7 @@ def load():
     L.rlrm_probe_random_gather.argtypes = [C.c_int, vp, i64, i32, i64, i32, vp, vp]
     L.rlrm_launch_count.argtypes = [vp]
     L.rlrm_launch_count.restype = i64
-    for name in ("rlrm_create", "rlrm_destroy", "rlrm_set_learner", "rlrm_set_sweep", "rlrm_reset", "rlrm_reset_at", "rlrm_select_action", "rlrm_step",
+    for name in ("rlrm_create", "rlrm_destroy", "rlrm_set_learner", "rlrm_set_sweep", "rlrm_set_exploration", "rlrm_reset", "rlrm_reset_at", "rlrm_select_action", "rlrm_step",
                  "rlrm_rm_step", "rlrm_rm_step_agent", "rlrm_mdp", "rlrm_value_iteration", "rlrm_update", "rlrm_train", "rlrm_train_host", "rlrm_evaluate", "rlrm_qlambda_materialize",
                  "rlrm_iterate", "rlrm_update_list", "rlrm_update_list_select", "rlrm_merge_replicas", "rlrm_stream_sync", "rlrm_probe_random_gather"):
         getattr(L, name).restype = C.c_int

@@ -19,6 +19,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <cmath>
 #include <new>
 
 #include "../../include/rlrm_b200.h"
@@ -60,6 +61,8 @@ struct rlrm_handle {
   int n_sweep;
   long long sweep_group;
   int sweep_lr_none;  // some setting has learning_rate = None (needs state.visits)
+  int softmax;        // rlrm_set_exploration(RLRM_EXPLORE_SOFTMAX): the SOFTMAX instantiations, specialised kernels skipped
+  double beta;        // 1 / temperature
 };
 
 // run STMT with T = float or double, whichever table type the handle was created for
@@ -519,6 +522,24 @@ extern "C" int rlrm_set_sweep(rlrm_handle_t* h, const rlrm_hyper_t* sets, int32_
   return RLRM_OK;
 }
 
+extern "C" int rlrm_set_exploration(rlrm_handle_t* h, int32_t kind, double temperature) {
+  if (!h) return fail(RLRM_ERR_ARG, "null handle");
+  if (kind != RLRM_EXPLORE_EPSILON_GREEDY && kind != RLRM_EXPLORE_SOFTMAX) return fail(RLRM_ERR_ARG, "rlrm_set_exploration: unknown kind");
+  if (kind == RLRM_EXPLORE_EPSILON_GREEDY) {
+    h->softmax = 0;
+    h->beta = 0.0;
+    return RLRM_OK;
+  }
+  const double beta = 1.0 / temperature;
+  if (!(temperature > 0.0) || !std::isfinite(temperature) || !std::isfinite(beta))
+    return fail(RLRM_ERR_ARG, "rlrm_set_exploration: the temperature must be finite and > 0, with a finite reciprocal");
+  // the shared learner's routes (persistent, cluster, propose + apply) select in kernels of their own
+  if (h->kp.shared_q) return fail(RLRM_ERR_UNSUPPORTED, "rlrm_set_exploration: softmax on a shared table is not supported");
+  h->softmax = 1;
+  h->beta = beta;
+  return RLRM_OK;
+}
+
 extern "C" int64_t rlrm_launch_count(const rlrm_handle_t* h) { return h ? (int64_t)h->launches : 0; }
 
 static DState dstate(const rlrm_state_t* st) {
@@ -603,8 +624,13 @@ extern "C" int rlrm_select_action(rlrm_handle_t* h, const rlrm_state_t* st, cons
   if (!actions_out) return fail(RLRM_ERR_ARG, "actions_out is null");
   CUDA_TRY(cudaSetDevice(h->device));
   const long long n = st->n_instances * h->kp.A;
-  if (h->kp.per_agent) RLRM_BY_T(h, select_kernel<true, T><<<blocks_for(n, 256), 256, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), draws, t, best, actions_out));
-  else RLRM_BY_T(h, select_kernel<false, T><<<blocks_for(n, 256), 256, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), draws, t, best, actions_out));
+#define RLRM_SEL(PA, SM) RLRM_BY_T(h, select_kernel<PA, T, SM><<<blocks_for(n, 256), 256, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), draws, t, best, actions_out, h->beta))
+  if (h->softmax) {
+    if (h->kp.per_agent) RLRM_SEL(true, true); else RLRM_SEL(false, true);
+  } else {
+    if (h->kp.per_agent) RLRM_SEL(true, false); else RLRM_SEL(false, false);
+  }
+#undef RLRM_SEL
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }
@@ -738,24 +764,31 @@ extern "C" int rlrm_update(rlrm_handle_t* h, const rlrm_state_t* st, const uint1
 }
 
 // SWEEP: the handle has per-group settings (h->d_sweep); every family takes them in its own kernel, fast paths included
-template <int ENV, bool SWEEP>
+// SOFTMAX: softmax exploration (h->softmax); only the generic and the Q(lambda) kernels have it, so the specialised ones are skipped
+template <int ENV, bool SWEEP, bool SOFTMAX>
 static void launch_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, int n_iters, int learn, uint32_t* trace, cudaStream_t s,
                          double* reward_out = nullptr) {
   const KP& kp = h->kp;
   const Sweep sw = sweep_of(h);
-  const bool fast_ok = reward_out == nullptr;  // the per-step reward output exists in the generic kernels only
+  const double beta = h->beta;
+  // the per-step reward output and softmax exploration exist in the generic kernels only
+  const bool fast_ok = reward_out == nullptr && !SOFTMAX;
   if (kp.algo == RLRM_ALGO_QLAMBDA && !st->e) {
     const long long ipw = 32 / (kp.qls_lg << kp.g_shift);  // instances per warp
     const long long qls_warps = (st->n_instances + ipw - 1) / ipw;
-    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, true, SWEEP><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
-    else RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, false, SWEEP><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
+    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, true, SWEEP, SOFTMAX><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw, beta));
+    else RLRM_BY_T(h, train_qlambda_sparse_kernel<ENV, T, false, SWEEP, SOFTMAX><<<blocks_for(qls_warps * 32, QLS_BLOCK), QLS_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw, beta));
   } else if (kp.algo == RLRM_ALGO_QLAMBDA) {
-    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_kernel<ENV, T, true, SWEEP><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
-    else RLRM_BY_T(h, train_qlambda_kernel<ENV, T, false, SWEEP><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw));
+    if (kp.per_agent) RLRM_BY_T(h, train_qlambda_kernel<ENV, T, true, SWEEP, SOFTMAX><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw, beta));
+    else RLRM_BY_T(h, train_qlambda_kernel<ENV, T, false, SWEEP, SOFTMAX><<<(unsigned)st->n_instances, kp.A * 32, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw, beta));
   } else {
     const long long threads = st->n_instances * kp.G;
     const unsigned grid = blocks_for(threads, TRAIN_BLOCK);
-#define RLRM_TRAIN(ALGO, PA) RLRM_BY_T(h, train_kernel<ENV, ALGO, PA, T, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw))
+#define RLRM_TRAIN(ALGO, PA)                                                                                                              \
+  do {                                                                                                                                    \
+    if (!SOFTMAX) RLRM_BY_T(h, train_kernel<ENV, ALGO, PA, T, SWEEP><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw, beta));    \
+    else RLRM_BY_T(h, train_kernel<ENV, ALGO, PA, T, SWEEP, true><<<grid, TRAIN_BLOCK, h->smem_bytes, s>>>(kp, dstate(st), t0, n_iters, learn, trace, reward_out, sw, beta)); \
+  } while (0)
     if (fast_ok && kp.algo == RLRM_ALGO_QRM && h->qrm4_fast && !st->visits) {
       const DState d = dstate(st);
 #define RLRM_QRM4(ST, LE, TR)                                                                                          \
@@ -834,6 +867,23 @@ static void launch_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, 
 #undef RLRM_TRAIN
   }
 }
+// the launch_train instantiation for the handle's environment, sweep and exploration (per-instance tables)
+static void launch_train_handle(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, int n_iters, int learn, uint32_t* trace, cudaStream_t s,
+                                double* reward_out = nullptr) {
+#define RLRM_LT(ENV)                                                                     \
+  do {                                                                                   \
+    if (h->d_sweep) {                                                                    \
+      if (h->softmax) launch_train<ENV, true, true>(h, st, t0, n_iters, learn, trace, s, reward_out);   \
+      else launch_train<ENV, true, false>(h, st, t0, n_iters, learn, trace, s, reward_out);             \
+    } else {                                                                             \
+      if (h->softmax) launch_train<ENV, false, true>(h, st, t0, n_iters, learn, trace, s, reward_out);  \
+      else launch_train<ENV, false, false>(h, st, t0, n_iters, learn, trace, s, reward_out);            \
+    }                                                                                    \
+  } while (0)
+  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) RLRM_LT(RLRM_ENV_FROZEN_LAKE);
+  else RLRM_LT(RLRM_ENV_OFFICE_WORLD);
+#undef RLRM_LT
+}
 
 extern "C" int rlrm_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0, int32_t n_iters, int32_t learn, uint32_t* trace,
                           void* stream) {
@@ -894,8 +944,8 @@ extern "C" int rlrm_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0,
           if (h->kp.algo == RLRM_ALGO_QRM) shared_propose_kernel<RLRM_ENV_OFFICE_WORLD, RLRM_ALGO_QRM><<<grid, SHARED_BLOCK, h->shared_smem_bytes, s>>>(h->kp, d, t0 + it, learn, tr);
           else shared_propose_kernel<RLRM_ENV_OFFICE_WORLD, RLRM_ALGO_QL><<<grid, SHARED_BLOCK, h->shared_smem_bytes, s>>>(h->kp, d, t0 + it, learn, tr);
         }
-      } else if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) launch_train<RLRM_ENV_FROZEN_LAKE, false>(h, st, t0 + it, 1, learn, tr, s);
-      else launch_train<RLRM_ENV_OFFICE_WORLD, false>(h, st, t0 + it, 1, learn, tr, s);
+      } else if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) launch_train<RLRM_ENV_FROZEN_LAKE, false, false>(h, st, t0 + it, 1, learn, tr, s);
+      else launch_train<RLRM_ENV_OFFICE_WORLD, false, false>(h, st, t0 + it, 1, learn, tr, s);
       LAUNCH_CHECK(h);
       if (learn) {
         apply_shared_kernel<<<blocks_for(h->kp.per_agent ? h->kp.sum4 : (long long)h->kp.A * h->kp.S4, 256), 256, 0, s>>>(h->kp, dstate(st));
@@ -904,13 +954,7 @@ extern "C" int rlrm_train(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t0,
     }
     return RLRM_OK;
   }
-  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) {
-    if (h->d_sweep) launch_train<RLRM_ENV_FROZEN_LAKE, true>(h, st, t0, n_iters, learn, trace, s);
-    else launch_train<RLRM_ENV_FROZEN_LAKE, false>(h, st, t0, n_iters, learn, trace, s);
-  } else {
-    if (h->d_sweep) launch_train<RLRM_ENV_OFFICE_WORLD, true>(h, st, t0, n_iters, learn, trace, s);
-    else launch_train<RLRM_ENV_OFFICE_WORLD, false>(h, st, t0, n_iters, learn, trace, s);
-  }
+  launch_train_handle(h, st, t0, n_iters, learn, trace, s);
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }
@@ -1046,13 +1090,7 @@ extern "C" int rlrm_iterate(rlrm_handle_t* h, const rlrm_state_t* st, uint64_t t
   }
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = (cudaStream_t)stream;
-  if (h->kp.env_kind == RLRM_ENV_FROZEN_LAKE) {
-    if (h->d_sweep) launch_train<RLRM_ENV_FROZEN_LAKE, true>(h, st, t, 1, learn, record, s, reward);
-    else launch_train<RLRM_ENV_FROZEN_LAKE, false>(h, st, t, 1, learn, record, s, reward);
-  } else {
-    if (h->d_sweep) launch_train<RLRM_ENV_OFFICE_WORLD, true>(h, st, t, 1, learn, record, s, reward);
-    else launch_train<RLRM_ENV_OFFICE_WORLD, false>(h, st, t, 1, learn, record, s, reward);
-  }
+  launch_train_handle(h, st, t, 1, learn, record, s, reward);
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }
@@ -1073,7 +1111,9 @@ static int update_list_impl(rlrm_handle_t* h, const rlrm_state_t* st, int64_t sl
     sa.state = sel->state; sa.best = sel->best; sa.epsilon = sel->epsilon; sa.seq = sel->seq;
     for (int j = 0; j < 4; j++) sa.draws[j] = sel->draws[j];
   }
-  RLRM_BY_T(h, update_list_kernel<T><<<1, (h->kp.algo == RLRM_ALGO_QLAMBDA && n > 0) ? 256 : 32, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), slot, n, experiences, sel, sa, sweep_of(h)));
+  const unsigned threads = (h->kp.algo == RLRM_ALGO_QLAMBDA && n > 0) ? 256 : 32;
+  if (h->softmax) RLRM_BY_T(h, update_list_kernel<T, true><<<1, threads, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), slot, n, experiences, sel, sa, sweep_of(h), h->beta));
+  else RLRM_BY_T(h, update_list_kernel<T, false><<<1, threads, 0, (cudaStream_t)stream>>>(h->kp, dstate(st), slot, n, experiences, sel, sa, sweep_of(h), h->beta));
   LAUNCH_CHECK(h);
   return RLRM_OK;
 }

@@ -251,6 +251,63 @@ __device__ __forceinline__ int select_action(const R& row, unsigned long long ex
   return a;
 }
 
+// Softmax exploration (rlrm_set_exploration; the rule is stated in include/rlrm_b200.h). rlrm_exp is a fixed sequence of IEEE-754
+// double operations for x <= 0 that the CPU oracle restates operation for operation (tests/softmax_oracle.c), so both sides get the
+// same bits: Cody-Waite reduction x = k*ln2 + r with |r| <= ln2/2, the degree-14 Taylor polynomial of exp(r) by Horner's rule with
+// FMA, and a scaling by 2^k built from its bit pattern (in two steps below 2^-1021, so that a subnormal result is rounded once).
+__device__ __forceinline__ double rlrm_exp(double x) {
+  if (x < -0x1.74910d52d3052p+9) return 0.0;  // below ln(2^-1075): exp(x) rounds to +0
+  const double k = rint(__dmul_rn(x, 0x1.71547652b82fep+0));  // log2(e)
+  double r = __fma_rn(-k, 0x1.62e42fefa39efp-1, x);            // ln2, high part
+  r = __fma_rn(-k, 0x1.abc9e3b39803fp-56, r);                  // ln2, low part
+  double p = 0x1.93974a8c07c9dp-37;                            // 1/14!, 1/13!, ..., 1/2!, 1, 1
+  p = __fma_rn(p, r, 0x1.6124613a86d09p-33);
+  p = __fma_rn(p, r, 0x1.1eed8eff8d898p-29);
+  p = __fma_rn(p, r, 0x1.ae64567f544e4p-26);
+  p = __fma_rn(p, r, 0x1.27e4fb7789f5cp-22);
+  p = __fma_rn(p, r, 0x1.71de3a556c734p-19);
+  p = __fma_rn(p, r, 0x1.a01a01a01a01ap-16);
+  p = __fma_rn(p, r, 0x1.a01a01a01a01ap-13);
+  p = __fma_rn(p, r, 0x1.6c16c16c16c17p-10);
+  p = __fma_rn(p, r, 0x1.1111111111111p-7);
+  p = __fma_rn(p, r, 0x1.5555555555555p-5);
+  p = __fma_rn(p, r, 0x1.5555555555555p-3);
+  p = __fma_rn(p, r, 0x1.0p-1);
+  p = __fma_rn(p, r, 1.0);
+  p = __fma_rn(p, r, 1.0);
+  const int ki = (int)k;  // -1075 .. 0
+  if (ki < -1021) return __dmul_rn(__dmul_rn(p, __longlong_as_double((long long)(ki + 54 + 1023) << 52)), 0x1.0p-54);
+  return __dmul_rn(p, __longlong_as_double((long long)(ki + 1023) << 52));
+}
+
+// Softmax selection on the row's first n_actions entries with beta = 1 / temperature: weights w_a = rlrm_exp((Q[a] - max) * beta),
+// cumulative sums C_j in action order, thresholds T_j = ceil(C_j / C_{n-1} * 2^32), action = #{j < n-1 : w1 >= T_j}. Zero
+// weights give empty intervals. best: the first argmax, exactly as select_action.
+template <typename R>
+__device__ __forceinline__ int select_softmax(const R& row, unsigned w1, double beta, bool best, unsigned n_actions) {
+  if (best) {
+    const unsigned w[4] = {0u, 0u, 0u, 0u};
+    return select_action(row, 0ull, w, true, n_actions);
+  }
+  const double q[4] = {(double)row.x, (double)row.y, (double)row.z, (double)row.w};
+  double m = q[0];
+#pragma unroll
+  for (int j = 1; j < 4; j++)
+    if ((unsigned)j < n_actions && q[j] > m) m = q[j];
+  double c[4], total = 0.0;
+#pragma unroll
+  for (int j = 0; j < 4; j++) {
+    if ((unsigned)j < n_actions) total = __dadd_rn(total, rlrm_exp(__dmul_rn(__dsub_rn(q[j], m), beta)));
+    c[j] = total;
+  }
+  int action = 0;
+#pragma unroll
+  for (int j = 0; j < 3; j++)
+    if ((unsigned)j + 1u < n_actions)
+      action += (unsigned long long)w1 >= (unsigned long long)ceil(__dmul_rn(__ddiv_rn(c[j], total), 4294967296.0));
+  return action;
+}
+
 __device__ __forceinline__ int slip_outcome(const KP& p, int intended, unsigned k) {
   int idx = 0;
 #pragma unroll

@@ -31,9 +31,9 @@ __global__ void __launch_bounds__(256) clear_traces_kernel(KP p, DState st, cons
   reinterpret_cast<typename RT<T>::row_t*>(st.e)[g] = RT<T>::zero_row();
 }
 
-template <bool PA, typename T>
+template <bool PA, typename T, bool SOFTMAX>  // SOFTMAX: softmax exploration with beta = 1 / temperature (see train_kernel)
 __global__ void __launch_bounds__(256) select_kernel(KP p_in, DState st, const unsigned* draws, unsigned long long t, int best,
-                                                    unsigned char* actions_out) {
+                                                    unsigned char* actions_out, double beta) {
   KP p = p_in;
   const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (k >= st.N * p.A) return;
@@ -50,7 +50,8 @@ __global__ void __launch_bounds__(256) select_kernel(KP p_in, DState st, const u
   } else {
     RLRM_PHILOX((unsigned)t, (unsigned)(t >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
   }
-  actions_out[k] = (unsigned char)select_action(row, explore_threshold(st.epsilon[k]), w, best != 0, p.n_actions);
+  actions_out[k] = (unsigned char)(SOFTMAX ? select_softmax(row, w[1], beta, best != 0, p.n_actions)
+                                           : select_action(row, explore_threshold(st.epsilon[k]), w, best != 0, p.n_actions));
 }
 
 __device__ __forceinline__ void store_rec(const DOut& o, long long k, const Rec& r) {
@@ -337,9 +338,9 @@ struct SelArgs {  // the input half of rlrm_select_req_t, passed by value (read 
   unsigned draws[4];
   unsigned seq;
 };
-template <typename T>
+template <typename T, bool SOFTMAX>  // SOFTMAX: the selection is softmax exploration with beta = 1 / temperature (see train_kernel)
 __global__ void __launch_bounds__(256) update_list_kernel(KP p, DState st, long long slot, int n, const rlrm_experience_t* ex,
-                                                         rlrm_select_req_t* sel, SelArgs sa, Sweep sw) {
+                                                         rlrm_select_req_t* sel, SelArgs sa, Sweep sw, double beta) {
   const long long i = slot / p.A;
   const int a = (int)(slot - i * p.A);
   KP pl = p;  // the slot's learner settings (a sweep handle's group); p itself stays in the constant bank
@@ -375,7 +376,9 @@ __global__ void __launch_bounds__(256) update_list_kernel(KP p, DState st, long 
   if (sel && threadIdx.x == 0) {
     const unsigned w[4] = {sa.draws[0], sa.draws[1], sa.draws[2], sa.draws[3]};
     const typename RT<T>::row_t row = load_row<T>(Q, min(sa.state, rows - 1u));
-    *reinterpret_cast<volatile unsigned*>(&sel->action) = (unsigned)select_action(row, explore_threshold(sa.epsilon), w, sa.best != 0, p.n_actions);
+    *reinterpret_cast<volatile unsigned*>(&sel->action) =
+        (unsigned)(SOFTMAX ? select_softmax(row, w[1], beta, sa.best != 0, p.n_actions)
+                           : select_action(row, explore_threshold(sa.epsilon), w, sa.best != 0, p.n_actions));
     __threadfence_system();
     *reinterpret_cast<volatile unsigned*>(&sel->done_seq) = sa.seq;
   }

@@ -6,9 +6,10 @@
 // PA = agents carry different reward machines: the warp's agent gets its own view of the parameters (a private copy); with
 // PA = false the parameter block stays in the constant bank
 // SWEEP: the block's instance takes its group's learner settings
-template <int ENV, typename T, bool PA, bool SWEEP>
+// SOFTMAX: softmax exploration with beta = 1 / temperature, the last parameter (see train_kernel)
+template <int ENV, typename T, bool PA, bool SWEEP, bool SOFTMAX>
 __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, unsigned long long t0, int n_iters, int learn,
-                                                           unsigned* trace, double* reward_out, Sweep sw) {
+                                                           unsigned* trace, double* reward_out, Sweep sw, double beta) {
   typedef RT<T> R;
   typedef typename R::row_t row_t;
   KP p_view, p_sw;  // p_sw: a sweep handle's learner settings, read only where they are used (ph; see train_ql_fast_kernel)
@@ -48,7 +49,7 @@ __global__ void __launch_bounds__(256) train_qlambda_kernel(KP p_in, DState st, 
     RLRM_PHILOX((unsigned)t, (unsigned)(t >> 32), p.instance_offset + (unsigned)i, (unsigned)a, p, w);
     __syncwarp();
     const row_t row = load_row<T>(Q, s.cell * p.nQ + s.rm);
-    const int action = select_action(row, explore_thr, w, learn == 0, p.n_actions);
+    const int action = SOFTMAX ? select_softmax(row, w[1], beta, learn == 0, p.n_actions) : select_action(row, explore_thr, w, learn == 0, p.n_actions);
     const unsigned before = s.cell;
     const bool first = (s.flags & RLRM_FLAG_FIRST) != 0;
     Rec r;
@@ -177,9 +178,9 @@ __device__ __forceinline__ void trace_flush(T* Q, const TraceList<T>& L, unsigne
                                // config 4's scenario with 1 / 2 / 4 agents): 1 agent 32 -> 8 lanes 1.82e9 -> 3.81e9, 2 agents 16 -> 8 lanes 3.05e9 -> 3.95e9;
                                // 4 lanes halve the rate everywhere (the visited entry's lookup needs a second round, a sweep waits for the longest of 8 lists)
 #endif
-template <int ENV, typename T, bool PA, bool SWEEP>
+template <int ENV, typename T, bool PA, bool SWEEP, bool SOFTMAX>
 __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in, DState st, unsigned long long t0, int n_iters, int learn,
-                                                                        unsigned* trace, double* reward_out, Sweep sw) {
+                                                                        unsigned* trace, double* reward_out, Sweep sw, double beta) {
   typedef RT<T> R;
   typedef typename R::row_t row_t;
   typedef typename R::pair_t pair_t;
@@ -247,7 +248,7 @@ __global__ void __launch_bounds__(QLS_BLOCK) train_qlambda_sparse_kernel(KP p_in
     row.y = __shfl_sync(FULL, mine, 1, LG);
     row.z = __shfl_sync(FULL, mine, 2, LG);
     row.w = __shfl_sync(FULL, mine, 3, LG);
-    const int action = select_action(row, explore_thr, w, learn == 0, p.n_actions);
+    const int action = SOFTMAX ? select_softmax(row, w[1], beta, learn == 0, p.n_actions) : select_action(row, explore_thr, w, learn == 0, p.n_actions);
     const unsigned before = s.cell;
     const bool first = (s.flags & RLRM_FLAG_FIRST) != 0;
     Rec r;

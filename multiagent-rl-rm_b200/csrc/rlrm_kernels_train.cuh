@@ -22,9 +22,15 @@
 
 // T = table arithmetic type (float: float32 tables; double: the reference's native float64 tables, see RT<T>)
 // SWEEP: the handle carries per-group learner settings (rlrm_set_sweep); every fused kernel takes the flag the same way
-template <int ENV, int ALGO, bool PA, typename T, bool SWEEP>
+// SOFTMAX: softmax exploration with beta = 1 / temperature (rlrm_set_exploration) instead of epsilon-greedy. It is an optional
+// trailing flag: the epsilon-greedy instantiations leave it out and keep the names and template arguments (train_kernel<ENV, ALGO,
+// PA, T, SWEEP>) by which profiles and the route tests identify them; the softmax ones are train_kernel<ENV, ALGO, PA, T, SWEEP,
+// true>. beta is the last parameter, so every other parameter sits where it was.
+template <int ENV, int ALGO, bool PA, typename T, bool SWEEP, bool... SOFTMAX_FLAG>
 __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_kernel(KP p_in, DState st, unsigned long long t0, int n_iters, int learn,
-                                                           unsigned* trace, double* reward_out, Sweep sw) {
+                                                           unsigned* trace, double* reward_out, Sweep sw, double beta) {
+  static_assert(sizeof...(SOFTMAX_FLAG) <= 1, "one optional SOFTMAX flag");
+  constexpr bool SOFTMAX = (false || ... || SOFTMAX_FLAG);
   typedef RT<T> R;
   typedef typename R::row_t row_t;
   KP p = p_in;
@@ -87,7 +93,7 @@ __global__ void __launch_bounds__(TRAIN_BLOCK, sizeof(T) == 4 ? 7 : 5) train_ker
         row = load_row<T>(Q, cur_idx);
         row_idx = carry ? cur_idx : 0xFFFFFFFFu;
       }
-      action = select_action(row, explore_thr, w, learn == 0, p.n_actions);
+      action = SOFTMAX ? select_softmax(row, w[1], beta, learn == 0, p.n_actions) : select_action(row, explore_thr, w, learn == 0, p.n_actions);
       const unsigned before = s.cell;
       const bool first = (s.flags & RLRM_FLAG_FIRST) != 0;
       agent_step<ENV>(p, tb, s, action, w[3], true, r);

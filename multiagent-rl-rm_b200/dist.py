@@ -72,10 +72,13 @@ def _default_engine_factory(compiled, n_local, device, **kw):
 
 class ShardedTrainer:
     def __init__(self, scenario: Scenario, n_instances_total: int, sync_every: Optional[int] = None, device=None,
-                 engine_factory: Callable = _default_engine_factory, group=None, sweep=None):
+                 engine_factory: Callable = _default_engine_factory, group=None, sweep=None, exploration: str = "epsilon_greedy",
+                 temperature: float = 1.0):
         """sweep: a hyper-parameter sweep over the whole batch (engine.Engine): setting g covers global instances
         [g * n_total / len(sweep), (g + 1) * n_total / len(sweep)). Settings are keyed on the global id, so every rank
-        uploads the same list and trains its shard's part of each group."""
+        uploads the same list and trains its shard's part of each group.
+        exploration / temperature: the engines' exploration (engine.Engine); the draws are keyed on the global id, so a
+        softmax run is the same whatever the number of ranks."""
         self.group = group
         self.world = dist.get_world_size(group) if dist.is_initialized() else 1
         self.rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -87,12 +90,13 @@ class ShardedTrainer:
         self.shared = bool(scenario.shared_q)
         self.sync_every = int(sync_every) if (self.shared and sync_every) else 0
         self.compiled = compile_scenario(scenario, instance_offset=self.offset)
+        kw = {} if exploration == "epsilon_greedy" else {"exploration": exploration, "temperature": temperature}
         if sweep is None:
-            self.engine = engine_factory(self.compiled, self.n_local, device)
+            self.engine = engine_factory(self.compiled, self.n_local, device, **kw)
         else:
             if self.n_total % len(sweep):
                 raise ValueError("n_instances_total must be a multiple of len(sweep)")
-            self.engine = engine_factory(self.compiled, self.n_local, device, sweep=sweep, sweep_group=self.n_total // len(sweep))
+            self.engine = engine_factory(self.compiled, self.n_local, device, sweep=sweep, sweep_group=self.n_total // len(sweep), **kw)
         self.t = 0
         self.syncs = 0
 

@@ -31,6 +31,8 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else t.data_ptr()
 
 
+EXPLORATIONS = {"epsilon_greedy": abi.EXPLORE_EPSILON_GREEDY, "softmax": abi.EXPLORE_SOFTMAX}
+
 SWEEP_KEYS = ("learning_rate", "gamma", "lambd", "epsilon_start", "epsilon_end", "epsilon_decay")
 
 
@@ -67,7 +69,7 @@ def sweep_settings(scenario, sweep) -> List[dict]:
 class Engine:
     def __init__(self, compiled: Compiled, n_instances: int, device="cuda:0", track_visits: bool = False,
                  with_stats: bool = True, qlambda_sparse: bool = False, host_control: bool = False, sweep=None,
-                 sweep_group: Optional[int] = None):
+                 sweep_group: Optional[int] = None, exploration: str = "epsilon_greedy", temperature: float = 1.0):
         """host_control: keep the small per-slot control state (slot words, epsilon, running return) in page-locked HOST
         memory instead of device memory. Page-locked memory is device-accessible under unified addressing, so the kernels
         read / write it in place and a host driver (the one-instance reference-shaped classes in envs.py) touches it through
@@ -78,7 +80,9 @@ class Engine:
         sweep: a hyper-parameter sweep, a list of dicts with keys among SWEEP_KEYS (missing keys come from the scenario).
         Setting g applies to the sweep_group instances with global ids [g * sweep_group, (g + 1) * sweep_group), global id =
         compiled instance_offset + local index; sweep_group defaults to n_instances // len(sweep), which must then divide
-        evenly. Every instance behaves bit for bit as in an engine built with its setting (rlrm_set_sweep)."""
+        evenly. Every instance behaves bit for bit as in an engine built with its setting (rlrm_set_sweep).
+        exploration: "epsilon_greedy" (the reference's QLearning.choose_action) or "softmax" with `temperature` (> 0), the
+        exactly specified softmax rule of rlrm_set_exploration; epsilon is still carried and decayed per slot, unread."""
         self.L = load()
         if not torch.cuda.is_available():
             raise RuntimeError("multiagent-rl-rm_b200 needs a CUDA device (no CPU fallback)")
@@ -108,6 +112,8 @@ class Engine:
             sets = (abi.Hyper * len(self.sweep))(*[abi.Hyper(-1.0 if s["learning_rate"] is None else s["learning_rate"], s["gamma"],
                                                              s["lambd"], s["epsilon_end"], s["epsilon_decay"]) for s in self.sweep])
             check(self.L.rlrm_set_sweep(self.h, sets, len(self.sweep), self.sweep_group))
+        self.exploration = self.temperature = None
+        self.set_exploration(exploration, temperature)
         n_slots = self.N * self.A
         n_tab = self.A if self.cfg.shared_q else n_slots
         tab_shape = (n_tab, self.S, 4)
@@ -174,6 +180,14 @@ class Engine:
 
     def set_learner(self, learning_rate, gamma, lambd=0.0):
         check(self.L.rlrm_set_learner(self.h, -1.0 if learning_rate is None else float(learning_rate), float(gamma), float(lambd)))
+
+    def set_exploration(self, exploration: str = "epsilon_greedy", temperature: float = 1.0):
+        """Exploration of every later selection (rlrm_set_exploration): "epsilon_greedy" or "softmax" at `temperature`."""
+        if exploration not in EXPLORATIONS:
+            raise ValueError(f"exploration must be one of {sorted(EXPLORATIONS)}")
+        softmax = exploration == "softmax"
+        check(self.L.rlrm_set_exploration(self.h, EXPLORATIONS[exploration], float(temperature) if softmax else 0.0))
+        self.exploration, self.temperature = exploration, (float(temperature) if softmax else None)
 
     def sync(self):
         """Wait for the work queued on the current stream (rlrm_stream_sync)."""
@@ -435,7 +449,8 @@ class Engine:
         1922-1925; see learners.QLearning.__getstate__ for that format); a batch of instances resumes from this instead."""
         out = {k: getattr(self, k).cpu() for k in self._STATE_TENSORS if getattr(self, k) is not None}
         out.update({"t": int(self.t), "n_instances": self.N, "n_agents": self.A, "state_space": self.S, "sparse": self.sparse,
-                    "sweep": None if self.sweep is None else [dict(s) for s in self.sweep], "sweep_group": self.sweep_group})
+                    "sweep": None if self.sweep is None else [dict(s) for s in self.sweep], "sweep_group": self.sweep_group,
+                    "exploration": self.exploration, "temperature": self.temperature})
         return out
 
     def load_state_dict(self, state: Dict[str, object]) -> None:
@@ -443,6 +458,8 @@ class Engine:
             raise ValueError("checkpoint was taken from a differently shaped engine")
         if (state.get("sweep"), state.get("sweep_group")) != (self.sweep, self.sweep_group):
             raise ValueError("checkpoint was taken from an engine with a different hyper-parameter sweep")
+        if (state.get("exploration", "epsilon_greedy"), state.get("temperature")) != (self.exploration, self.temperature):
+            raise ValueError("checkpoint was taken from an engine with a different exploration setting")
         for k in self._STATE_TENSORS:
             mine = getattr(self, k)
             if (mine is None) != (k not in state):
